@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — one JSON line per run (driver contract, "tier" reading).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 A step = one search() of the whole 10k-query batch through the library's C ABI.
   value   QPS with queries resident in HBM (device-timed, CUDA events, L2 flushed between steps)
@@ -17,8 +17,12 @@ codes), n_probes 48, exact refine of 2k candidates, batch 10k, k 10; 51 GB of ve
 f16|u8|f32; N > 1 = index sharded by IVF list, one all-gather of partial top-k), ivf_pq_c2 (BASELINE configs[2]: 10M x 128, n_lists
 1024, n_probes 64), brute_force (configs[1], 1M x 128, bit-exact vs the oracle), cagra (configs[3], 10M x 96, degree 64, itopk 64;
 --walk-bits 32|16), ivf_flat (configs[4] scaled to 10M, list-sharded for N > 1).  --no-cpu skips the CPU baseline, --no-aux the
-secondary harder-data point.  Recall denominators come from our exact brute force, itself checked against the oracle on a slice
-of the same tensors (config.ground_truth_check); a failed check or recall < 0.95 adds PARITY_FAILED to the line.
+secondary harder-data point.  --dump-outputs DIR writes what the last timed step returned (distances.npy, neighbors.npy) so
+that two builds can be compared output for output: the inputs are generated from fixed seeds, and index builds sum and order
+in input order, not in atomic order (tests/test_build_determinism_gpu.py asserts equal indexes and equal search answers for
+two builds of one input).  Recall denominators come from
+our exact brute force, itself checked against the oracle on a slice of the same tensors (config.ground_truth_check); a failed
+check or recall < 0.95 adds PARITY_FAILED to the line.
 """
 from __future__ import annotations
 
@@ -172,6 +176,9 @@ class BruteForceWorkload:
     def cpu_baseline(self, budget_s=20.0):
         return cpu_baseline_on_slice(self.dataset, self.queries, self.k, budget_s, "the same search, answered on the host")
 
+    def outputs(self):
+        return {"distances": self.distances, "neighbors": self.neighbors}
+
     def check(self):
         import oracle
         qs = self.queries[:32].cpu().numpy()
@@ -180,9 +187,9 @@ class BruteForceWorkload:
         return bool(ok)
 
 
-def cpu_exact_knn_rate(ds_rows, qs, k, budget_s, what, n_total=None):
+def cpu_exact_knn_rate(ds_rows, qs, k, budget_s, what, n_total=None, repeats=3):
     """CPU baseline: exact fp32 kNN with the oracle port on ALL host threads, in a separate process with pinned OpenMP
-    threads (oracle/cpu_baseline.py), 3 timed repeats after a warm-up, median reported.  `ds_rows` may be a ROW SLICE of the
+    threads (oracle/cpu_baseline.py), `repeats` timed repeats after a warm-up, median reported.  `ds_rows` may be a ROW SLICE of the
     workload's dataset (host RAM / time bound): the rate is then scaled by rows(slice) / n_total — exact kNN cost is linear
     in the rows scanned — and the sample says so."""
     import tempfile
@@ -196,16 +203,16 @@ def cpu_exact_knn_rate(ds_rows, qs, k, budget_s, what, n_total=None):
     script = os.path.join(ROOT, "oracle", "cpu_baseline.py")
     try:
         np.save(f_ds, ds_rows)
-        # size the query sample from a short probe run so that warm-up + 3 repeats take ~budget_s
+        # size the query sample from a short probe run so that warm-up + repeats take ~budget_s
         np.save(f_q, np.ascontiguousarray(qs[:16]))
         r = subprocess.run([sys.executable, script, f_ds, f_q, str(k), "1"], env=env, capture_output=True, text=True, timeout=600)
         probe = json.loads(r.stdout.strip().splitlines()[-1])
         rate = max(probe["probe_rates_qps"].values())
         # at least one full 256-query block: the workload is a 10k-query BATCH, and a skinny GEMM (a few dozen queries per pass
         # over the rows) would measure the host's memory bandwidth, not what a tuned CPU brute force does with the batch
-        m = int(min(len(qs), max(256, budget_s / 4.0 * rate)))
+        m = int(min(len(qs), max(256, budget_s / (repeats + 1.0) * rate)))
         np.save(f_q, np.ascontiguousarray(qs[:m]))
-        r = subprocess.run([sys.executable, script, f_ds, f_q, str(k), "3", probe["formulation"]], env=env, capture_output=True,
+        r = subprocess.run([sys.executable, script, f_ds, f_q, str(k), str(repeats), probe["formulation"]], env=env, capture_output=True,
                            text=True, timeout=900)
         out = json.loads(r.stdout.strip().splitlines()[-1])
     finally:
@@ -218,9 +225,9 @@ def cpu_exact_knn_rate(ds_rows, qs, k, budget_s, what, n_total=None):
     form = "blocked SGEMM + top-k (oracle.knn_blocked)" if out["formulation"] == "blocked" else "sequential-fmaf scan (oracle.knn, OpenMP)"
     sample = (f"{m} queries, exact fp32 kNN over {n_slice} rows"
               + (f" (a row slice of the {n_total}-row dataset; rate scaled by {scale:.4g}: cost is linear in rows)" if n_slice != n_total else "")
-              + f" ({what}); {form}; separate process, OMP_PROC_BIND=spread OMP_PLACES=threads; 3 repeats after warm-up: "
-              f"median {qps[1]:.3g}, min {qps[-1]:.3g}, max {qps[0]:.3g} q/s")
-    return {"value": qps[1], "unit": "queries/s", "cores": threads, "kind": "port", "sample": sample,
+              + f" ({what}); {form}; separate process, OMP_PROC_BIND=spread OMP_PLACES=threads; {repeats} repeats after warm-up: "
+              f"median {qps[len(qps) // 2]:.3g}, min {qps[-1]:.3g}, max {qps[0]:.3g} q/s")
+    return {"value": qps[len(qps) // 2], "unit": "queries/s", "cores": threads, "kind": "port", "sample": sample,
             "repeats_qps": qps}
 
 
@@ -406,6 +413,11 @@ class IvfPqWorkload:
     def units(self):
         return self.nq
 
+    def outputs(self):
+        if self.sharded is not None:
+            return {"distances": self.final_d, "neighbors": self.final_i}
+        return {"distances": self.distances, "neighbors": self.neighbors}
+
     def check(self):
         nb = self.final_i if self.sharded is not None else self.neighbors
         hit = (nb.unsqueeze(2) == self.gt.unsqueeze(1)).any(dim=2).float().mean().item()
@@ -537,6 +549,9 @@ class CagraWorkload:
     def units(self):
         return self.nq
 
+    def outputs(self):
+        return {"distances": self.distances, "neighbors": self.neighbors}
+
     def check(self):
         nb = self.neighbors.to(torch.int64)
         self.recall = (nb.unsqueeze(2) == self.gt.unsqueeze(1)).any(dim=2).float().mean().item()
@@ -633,6 +648,9 @@ class IvfFlatWorkload:
     def units(self):
         return self.nq
 
+    def outputs(self):
+        return {"distances": self.final_d, "neighbors": self.final_i}
+
     def check(self):
         self.recall = (self.final_i.unsqueeze(2) == self.gt.unsqueeze(1)).any(dim=2).float().mean().item()
         return self.recall >= 0.95 and (self.gt_check is None or self.gt_check["ok"])
@@ -697,6 +715,29 @@ def ncu_traffic(workload, wl):
     if not ent or ent.get("n") != getattr(wl, "n", None) or ent.get("world", 1) != getattr(wl, "world", 1):
         return None
     return ent.get("dram_bytes_per_launch")
+
+
+DUMP_LIMIT_BYTES = 60 << 20   # array bytes of --dump-outputs: under 64 MB in all with the .npy headers
+
+
+def dump_outputs(outputs, out_dir):
+    """Writes each output of the timed search as out_dir/<name>.npy: floating-point values as float32, ids as float64 (exact
+    below 2**53).  Above DUMP_LIMIT_BYTES in all, every array keeps the same fixed, seeded sample of query rows, whose row
+    numbers go to rows.npy."""
+    arrays = {}
+    for name, t in outputs.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a.astype(np.float32 if a.dtype.kind == "f" and a.itemsize <= 4 else np.float64)
+    n = next(iter(arrays.values())).shape[0]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        keep = int(DUMP_LIMIT_BYTES // (total / n + 8))
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def launches():
@@ -797,6 +838,8 @@ def run_ours(args):
         n_launch = launches() - l0
         lib.cuvsB200TimingEnable(0)
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl.outputs(), args.dump_outputs)
     cnt = C.c_int(0)
     kernel_ms_total = lib.cuvsB200TimingTotalMs(wl.timing_section.encode(), C.byref(cnt))
     kernel_ms = kernel_ms_total / max(cnt.value, 1)
@@ -850,9 +893,9 @@ def harder_data_point(args, res, timed):
     for _ in range(3):
         wl.step(res)
     res.sync()
-    ms = timed(wl.step, 5)
+    ms = timed(wl.step, args.steps)
     ok = wl.check()
-    return {"workload": wl.name, "data": "rank-32 gaussian manifold + 0.05 noise", "qps": wl.units() * 5 / (ms * 1e-3),
+    return {"workload": wl.name, "data": "rank-32 gaussian manifold + 0.05 noise", "qps": wl.units() * args.steps / (ms * 1e-3),
             "recall_at_10": wl.recall, "ok": bool(ok)}
 
 
@@ -882,15 +925,16 @@ def run_reference(args):
         ds = gen_manifold(rows, d, 1234, rank=rk, device=dev)   # == the first `rows` rows of the GPU arm's dataset
         qs = gen_manifold(1024, d, 1234 + 3087, rank=rk, device=dev)
         name = f"{wl} {n // 1_000_000}M x {d} f32 workload, answered by exact CPU kNN (the reference has no CPU {wl} search)"
-    budget = max(8.0, 12.0 * max(args.steps, 1) / 3.0)
-    cb = cpu_exact_knn_rate(ds.cpu().numpy(), qs.cpu().numpy(), k, budget, "same tensors as the GPU arm", n_total=n)
+    budget = max(8.0, 12.0 * args.steps / 3.0)
+    cb = cpu_exact_knn_rate(ds.cpu().numpy(), qs.cpu().numpy(), k, budget, "same tensors as the GPU arm", n_total=n,
+                            repeats=args.steps)
     v = cb["value"]
     print(json.dumps({
         "impl": "reference", "metric": METRIC_NAME, "value": v, "unit": "queries/s", "n_gpus": int(os.environ.get("WORLD_SIZE", "1")),
-        "steps": 3, "warmup": 1, "ms_per_step": None, "higher_is_better": True, "scaling": "strong",
+        "steps": args.steps, "warmup": 1, "ms_per_step": None, "higher_is_better": True, "scaling": "strong",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": name, "n": n, "dim": d, "batch": nq, "k": k, "metric": "sqeuclidean", "recall_at_10": 1.0,
-                   "note": "steps/warmup: the CPU arm always runs 1 warm-up + 3 timed repeats of a bounded query sample (median reported)"},
+                   "note": "steps/warmup: the CPU arm runs 1 warm-up + --steps timed repeats of a bounded query sample (median reported)"},
         "cpu_baseline": cb,
         "e2e": {"value": v, "unit": "queries/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }))
@@ -924,7 +968,13 @@ def main():
     ap.add_argument("--no-aux", action="store_true", help="skip the secondary harder-data (rank-32, 10M) measurement of the ivf_pq line")
     ap.add_argument("--itopk", type=int, default=0)
     ap.add_argument("--degree", type=int, default=0)
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm only times the CPU search)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -30,6 +30,7 @@
 #include "npy_io.hpp"
 #include "ptx_sm100.cuh"
 #include "exact.cuh"
+#include "ivf_lists.cuh"
 #include "select_k.cuh"
 #include "timing.hpp"
 
@@ -772,16 +773,25 @@ __global__ void knn_to_graph_kernel(const int64_t* __restrict__ knn, int64_t n, 
   (void)keep;
 }
 
-__global__ void reverse_edges_kernel(const uint32_t* __restrict__ fwd, int64_t n, int degree, int keep, uint32_t* __restrict__ rev,
-                                     uint32_t* __restrict__ rev_cnt, int rev_cap)
+// each of the first `keep` forward edges (u, v) as (target v, source u), in source order
+__global__ void forward_edges_kernel(const uint32_t* __restrict__ fwd, int64_t n, int degree, int keep, uint32_t* __restrict__ tgt,
+                                     uint32_t* __restrict__ src)
 {
   int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
   if (t >= n * keep) return;
-  int64_t u = t / keep;
-  int r     = static_cast<int>(t % keep);
-  uint32_t v = fwd[u * degree + r];
-  uint32_t slot = atomicAdd(&rev_cnt[v], 1u);
-  if (slot < static_cast<uint32_t>(rev_cap)) rev[static_cast<int64_t>(v) * rev_cap + slot] = static_cast<uint32_t>(u);
+  tgt[t] = fwd[(t / keep) * degree + t % keep];
+  src[t] = static_cast<uint32_t>(t / keep);
+}
+
+// reverse edges of node v: its sources u in ascending order (edges grouped by target, stably), the first rev_cap kept
+__global__ void reverse_edges_kernel(const uint32_t* __restrict__ src, const int64_t* __restrict__ start, int64_t n,
+                                     uint32_t* __restrict__ rev, uint32_t* __restrict__ rev_cnt, int rev_cap)
+{
+  int64_t v = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (v >= n) return;
+  const int64_t cnt = start[v + 1] - start[v];
+  for (int64_t slot = 0; slot < cnt && slot < rev_cap; ++slot) rev[v * rev_cap + slot] = src[start[v] + slot];
+  rev_cnt[v] = static_cast<uint32_t>(cnt);
 }
 
 // final row = first `keep` forward edges, then reverse edges not already present, then remaining forward edges
@@ -1140,7 +1150,7 @@ cuvsError_t cuvsCagraBuild(cuvsResources_t res, cuvsCagraIndexParams_t params, D
     else build_knn_graph_ivf(res, r, data, n, idx->dim, idx->metric, kk, knn.data());
     // ---- self-free neighbour rows, detour pruning, reverse-edge augmentation
     dbuf<uint32_t> nbr(static_cast<size_t>(n) * di, r->stream);
-    count_launch(5);
+    count_launch(4);
     knn_to_graph_kernel<<<blocks_for(n, 128), 128, 0, r->stream>>>(knn.data(), n, kk, di, nbr.data(), di);
     dbuf<uint32_t> counts(static_cast<size_t>(n) * di, r->stream);
     detour_count_kernel<<<static_cast<unsigned>(n), 128, sizeof(uint32_t) * 2 * di, r->stream>>>(nbr.data(), n, di, counts.data());
@@ -1149,8 +1159,16 @@ cuvsError_t cuvsCagraBuild(cuvsResources_t res, cuvsCagraIndexParams_t params, D
     const int keep    = std::max(1, degree / 2);
     const int rev_cap = degree;
     dbuf<uint32_t> rev(static_cast<size_t>(n) * rev_cap, r->stream), rev_cnt(static_cast<size_t>(n), r->stream);
-    B2_CUDA(cudaMemsetAsync(rev_cnt.data(), 0, sizeof(uint32_t) * n, r->stream));
-    reverse_edges_kernel<<<blocks_for(n * keep, 256), 256, 0, r->stream>>>(fwd.data(), n, degree, keep, rev.data(), rev_cnt.data(), rev_cap);
+    dbuf<uint32_t> src(static_cast<size_t>(n) * keep, r->stream);
+    dbuf<int64_t> start;
+    {
+      dbuf<uint32_t> tgt(static_cast<size_t>(n) * keep, r->stream);
+      count_launch();
+      forward_edges_kernel<<<blocks_for(n * keep, 256), 256, 0, r->stream>>>(fwd.data(), n, degree, keep, tgt.data(), src.data());
+      group_by_key(r->stream, tgt, src, n, start);
+    }
+    count_launch();
+    reverse_edges_kernel<<<blocks_for(n, 256), 256, 0, r->stream>>>(src.data(), start.data(), n, rev.data(), rev_cnt.data(), rev_cap);
     idx->graph_own.alloc(static_cast<size_t>(n) * degree);
     merge_graph_kernel<<<blocks_for(n, 128), 128, 0, r->stream>>>(fwd.data(), rev.data(), rev_cnt.data(), n, degree, keep, rev_cap, idx->graph_own.data());
     B2_CUDA(cudaGetLastError());

@@ -2,6 +2,7 @@
 #include "ivf_common.cuh"
 
 #include "exact.cuh"
+#include "ivf_lists.cuh"
 #include "select_k.cuh"
 #include "timing.hpp"
 
@@ -423,26 +424,33 @@ __global__ void strided_init_kernel(const float* __restrict__ x, int64_t n, int 
   centers[t]  = x[row * d + (t % d)];
 }
 
-__global__ void accumulate_kernel(const float* __restrict__ x, int64_t n, int d, const uint32_t* __restrict__ labels,
-                                  const float* __restrict__ weights, float* __restrict__ sums, float* __restrict__ counts)
+// one block per cluster: thread (column j, row lane r) sums the member rows r, r + R, ... in row order, and the R partial
+// sums are added in lane order, so the result does not depend on scheduling (same input, same centres, run after run)
+__global__ void segment_centers_kernel(const float* __restrict__ x, int d, int dp, const uint32_t* __restrict__ order,
+                                       const int64_t* __restrict__ start, const float* __restrict__ weights,
+                                       float* __restrict__ sums, float* __restrict__ counts, float* __restrict__ centers)
 {
-  // one warp per row; lanes stride over d
-  int64_t row = (blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5;
-  int lane    = threadIdx.x & 31;
-  if (row >= n) return;
-  uint32_t l = labels[row];
-  float w    = weights ? weights[row] : 1.0f;
-  for (int c = lane; c < d; c += 32) atomicAdd(&sums[static_cast<int64_t>(l) * d + c], w * x[row * d + c]);
-  if (lane == 0) atomicAdd(&counts[l], w);
-}
-
-__global__ void finalize_centers_kernel(const float* __restrict__ sums, const float* __restrict__ counts, int k, int d,
-                                        float* __restrict__ centers)
-{
-  int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (t >= static_cast<int64_t>(k) * d) return;
-  float c = counts[t / d];
-  if (c > 0.f) centers[t] = sums[t] / c;
+  extern __shared__ float part[];  // [R][dp] column partials, then [R] weight partials
+  const int64_t l = blockIdx.x;
+  const int j = threadIdx.x % dp, r = threadIdx.x / dp, R = blockDim.x / dp;
+  float acc = 0.f, wacc = 0.f;
+  for (int64_t p = start[l] + r; p < start[l + 1]; p += R) {
+    const int64_t row = order[p];
+    const float w     = weights ? weights[row] : 1.0f;
+    if (j < d) acc += w * x[row * d + j];
+    wacc += w;
+  }
+  part[r * dp + j] = acc;
+  if (j == 0) part[R * dp + r] = wacc;
+  __syncthreads();
+  if (r != 0) return;
+  float sum = 0.f, cnt = 0.f;
+  for (int q = 0; q < R; ++q) { sum += part[q * dp + j]; cnt += part[R * dp + q]; }
+  if (j < d) {
+    sums[l * d + j] = sum;
+    if (cnt > 0.f) centers[l * d + j] = sum / cnt;
+  }
+  if (j == 0) counts[l] = cnt;
 }
 
 __device__ __forceinline__ uint64_t mix64(uint64_t z)
@@ -697,11 +705,16 @@ bool merge_probe_candidates(cudaStream_t s, const float* cs, const uint32_t* cp,
 void update_centers(cudaStream_t s, const float* x, int64_t n, int d, const uint32_t* labels, const float* weights, int k,
                     float* centers, float* sums_ws, float* counts_ws)
 {
-  B2_CUDA(cudaMemsetAsync(sums_ws, 0, sizeof(float) * static_cast<size_t>(k) * d, s));
-  B2_CUDA(cudaMemsetAsync(counts_ws, 0, sizeof(float) * k, s));
-  count_launch(2);
-  accumulate_kernel<<<blocks_for(n * 32, 256), 256, 0, s>>>(x, n, d, labels, weights, sums_ws, counts_ws);
-  finalize_centers_kernel<<<blocks_for(static_cast<int64_t>(k) * d, 256), 256, 0, s>>>(sums_ws, counts_ws, k, d, centers);
+  B2_EXPECTS(d >= 1 && d <= 1024, "update_centers: dim %d is out of range", d);
+  dbuf<uint32_t> keys(static_cast<size_t>(n), s), order;
+  B2_CUDA(cudaMemcpyAsync(keys.data(), labels, sizeof(uint32_t) * n, cudaMemcpyDeviceToDevice, s));
+  iota_u32(s, order, n);
+  dbuf<int64_t> start;
+  group_by_key(s, keys, order, k, start);
+  const int dp = (d + 31) / 32 * 32, R = std::max(1, 512 / dp);
+  count_launch();
+  segment_centers_kernel<<<static_cast<unsigned>(k), R * dp, sizeof(float) * (R * dp + R), s>>>(x, d, dp, order.data(), start.data(),
+                                                                                                 weights, sums_ws, counts_ws, centers);
   B2_CUDA(cudaGetLastError());
 }
 

@@ -95,7 +95,7 @@ bool merge_probe_candidates(cudaStream_t s, const float* cs, const uint32_t* cp,
 void kmeans_train(resources* res, const float* x, int64_t n, int d, int k, int n_iters, float* centers,
                   bool init_from_data, bool balance, double* inertia, int* iters_done, double tol = 0.0);
 
-/** Sum of member rows and member counts per label (fp32 atomics), then centers = sums / counts where counts > 0. */
+/** Sum of member rows and member counts per label (in row order: deterministic), then centers = sums / counts where counts > 0. */
 void update_centers(cudaStream_t s, const float* x, int64_t n, int d, const uint32_t* labels, const float* weights,
                     int k, float* centers, float* sums_ws /*[k*d]*/, float* counts_ws /*[k]*/);
 

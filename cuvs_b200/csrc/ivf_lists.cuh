@@ -36,6 +36,16 @@ struct list_layout {
 void place_rows(cudaStream_t s, const uint32_t* labels, int64_t n, const list_layout& layout,
                 const std::vector<int64_t>& base_fill, int64_t* dst_rows);
 
+/**
+ * Deterministic grouping: sorts the pairs (keys[i], values[i]) stably by key, in place (on return both buffers hold the sorted
+ * pairs; the stable order keeps the input order inside a key), and sets start[g] = the first position of key g
+ * (n_groups + 1 entries, start[n_groups] = n).  Sums taken over a group in this order, or ranks taken inside it, do not
+ * depend on thread scheduling, unlike atomics.  Transient device memory: 8 bytes per item (the radix sort's second key and
+ * value buffers) + 8 bytes per group + CUB's small temporary storage.
+ */
+void group_by_key(cudaStream_t s, dbuf<uint32_t>& keys, dbuf<uint32_t>& values, int64_t n_groups, dbuf<int64_t>& start);
+/** v = 0, 1, ..., n - 1 (n < 2^32: larger inputs are rejected). */
+void iota_u32(cudaStream_t s, dbuf<uint32_t>& v, int64_t n);
 /** counts[l] = number of rows with that label (host vector, synchronises the stream). */
 std::vector<int64_t> count_labels(cudaStream_t s, const uint32_t* labels, int64_t n, int64_t n_lists);
 

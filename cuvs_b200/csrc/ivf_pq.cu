@@ -180,18 +180,38 @@ __global__ void __launch_bounds__(128) pq_assign_kernel(const float* __restrict_
   codes[o * pq_dim + sub] = static_cast<uint8_t>(bc);
 }
 
-__global__ void pq_accumulate_kernel(const float* __restrict__ resid, int64_t n, int rot_dim, int pq_dim, int pq_len, int book,
-                                     const uint8_t* __restrict__ codes, int per_cluster, const uint32_t* __restrict__ labels,
-                                     float* __restrict__ sums, float* __restrict__ counts)
+// codebook entry (book b, code) of every (row, subspace) item: key b * book + code
+__global__ void pq_keys_kernel(int64_t n, int pq_dim, int book, const uint8_t* __restrict__ codes, int per_cluster,
+                               const uint32_t* __restrict__ labels, uint32_t* __restrict__ keys)
 {
   int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
   if (t >= n * pq_dim) return;
-  int64_t r = t / pq_dim;
-  int sub   = static_cast<int>(t % pq_dim);
-  int code  = codes[t];
-  int64_t b = per_cluster ? labels[r] : sub;
-  for (int j = 0; j < pq_len; ++j) atomicAdd(&sums[(b * pq_len + j) * book + code], resid[r * rot_dim + sub * pq_len + j]);
-  atomicAdd(&counts[b * book + code], 1.0f);
+  const int64_t b = per_cluster ? labels[t / pq_dim] : t % pq_dim;
+  keys[t]         = static_cast<uint32_t>(b * book + codes[t]);
+}
+
+// one warp per codebook entry: lanes stride over its items in item order and the lane sums are combined by a fixed shuffle
+// tree, so the sums do not depend on scheduling (same input, same codebooks, run after run)
+__global__ void pq_segment_sums_kernel(const float* __restrict__ resid, int rot_dim, int pq_dim, int pq_len, int book,
+                                       int64_t n_entries, const uint32_t* __restrict__ order, const int64_t* __restrict__ start,
+                                       float* __restrict__ sums, float* __restrict__ counts)
+{
+  const int64_t g = (blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x) >> 5;
+  const int lane  = threadIdx.x & 31;
+  if (g >= n_entries) return;
+  const int64_t b = g / book, s0 = start[g], s1 = start[g + 1];
+  const int code  = static_cast<int>(g % book);
+  for (int j = 0; j < pq_len; ++j) {
+    float acc = 0.f;
+    for (int64_t p = s0 + lane; p < s1; p += 32) {
+      const int64_t t = order[p];
+      acc += resid[(t / pq_dim) * rot_dim + (t % pq_dim) * pq_len + j];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) sums[(b * pq_len + j) * book + code] = acc;
+  }
+  if (lane == 0) counts[g] = static_cast<float>(s1 - s0);
 }
 
 __global__ void pq_finalize_kernel(float* __restrict__ pq_centers, const float* __restrict__ sums, const float* __restrict__ counts,
@@ -635,16 +655,19 @@ void train_codebooks(resources* res, ivf_pq_index& idx, const float* resid, cons
   count_launch();
   pq_init_kernel<<<blocks_for(nb * book, 128), 128, 0, s>>>(idx.pq_centers.data(), nb, idx.pq_len, book, resid, n, idx.rot_dim, idx.pq_dim);
   dbuf<uint8_t> codes(static_cast<size_t>(n) * idx.pq_dim, s);
+  dbuf<uint32_t> keys(static_cast<size_t>(n) * idx.pq_dim, s), order;
+  dbuf<int64_t> start;
   dbuf<float> sums(static_cast<size_t>(nb) * idx.pq_len * book, s), counts(static_cast<size_t>(nb) * book, s);
   const size_t smem = static_cast<size_t>(idx.pq_len) * book * sizeof(float);
   for (int it = 0; it < n_iters; ++it) {
-    count_launch(3);
+    count_launch(4);
     pq_assign_kernel<<<dim3(blocks_for(n, 128), idx.pq_dim), 128, smem, s>>>(resid, n, idx.rot_dim, idx.pq_dim, idx.pq_len, book,
                                                                                idx.pq_centers.data(), per_cl, labels, codes.data(), nullptr);
-    B2_CUDA(cudaMemsetAsync(sums.data(), 0, sums.size() * sizeof(float), s));
-    B2_CUDA(cudaMemsetAsync(counts.data(), 0, counts.size() * sizeof(float), s));
-    pq_accumulate_kernel<<<blocks_for(n * idx.pq_dim, 256), 256, 0, s>>>(resid, n, idx.rot_dim, idx.pq_dim, idx.pq_len, book, codes.data(),
-                                                                           per_cl, labels, sums.data(), counts.data());
+    pq_keys_kernel<<<blocks_for(n * idx.pq_dim, 256), 256, 0, s>>>(n, idx.pq_dim, book, codes.data(), per_cl, labels, keys.data());
+    iota_u32(s, order, n * idx.pq_dim);
+    group_by_key(s, keys, order, nb * book, start);
+    pq_segment_sums_kernel<<<blocks_for(nb * book * 32, 256), 256, 0, s>>>(resid, idx.rot_dim, idx.pq_dim, idx.pq_len, book, nb * book,
+                                                                            order.data(), start.data(), sums.data(), counts.data());
     pq_finalize_kernel<<<blocks_for(nb * book, 128), 128, 0, s>>>(idx.pq_centers.data(), sums.data(), counts.data(), nb, idx.pq_len, book,
                                                                    resid, n, idx.rot_dim, idx.pq_dim, it, it == n_iters - 1);
     B2_CUDA(cudaGetLastError());

@@ -5,8 +5,8 @@
 //   kernel (kmeans_common.cuh:60-84) and runs cuBLAS GEMM into an n x k fp32 matrix + reduce_min_kernel
 //   (unfused_distance_nn.cuh:54-118), i.e. n*k*4 bytes written and read back through HBM per iteration.
 // Here the assignment is the tcgen05 scan kernel with its fused top-1 epilogue (ivf_common.cu: assign_nearest):
-// the n x k score block lives in TMEM only.  Lloyd iterations, centroid update (fp32 atomics) and the inertia
-// reduction are plain CUDA; C wrapper semantics follow c/src/cluster/kmeans.cpp.
+// the n x k score block lives in TMEM only.  Lloyd iterations, centroid update (per-cluster sums in row order, so the same
+// input gives the same centroids) and the inertia reduction are plain CUDA; C wrapper semantics follow c/src/cluster/kmeans.cpp.
 #include "common.hpp"
 #include "exact.cuh"
 #include "ivf_common.cuh"

@@ -6,6 +6,8 @@ harness (dataset -> build -> batched search -> recall -> Google-Benchmark-style 
 test-only CPU backend whose searcher is the oracle's exact kNN (test infrastructure; the product backend serves GPU algorithms
 only and never imports the oracle)."""
 import importlib
+import inspect
+import itertools
 import json
 import os
 import sys
@@ -15,6 +17,7 @@ import pytest
 
 import oracle
 from cuvs_b200 import bench_backend as bb
+from oracle.make_golden_cuvs_bench import BUILD_RESULT, SEARCH_RESULT, recall_inputs
 
 REF_PKG = "/root/reference/python/cuvs_bench"
 
@@ -54,6 +57,11 @@ def _c0_dataset_with_the_reference_ground_truth():
                       groundtruth_neighbors=np.array(case["ids"]), distance_metric="euclidean")
 
 
+def _reference_interface():
+    """What the reference's benchmark package defines and computes, recorded by oracle/make_golden_cuvs_bench.py."""
+    return json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cuvs_bench_interface.json")))
+
+
 def test_c0_harness_recall_against_the_reference_cpu_ground_truth():
     ds = _c0_dataset_with_the_reference_ground_truth()
     recs = bb.run_config({"name": "cpu_exact", "groups": {"base": {"build": {}, "search": {}}}}, ds, k=10, batch_size=50,
@@ -75,13 +83,7 @@ def test_c0_plumbing_10k_x_128_k10_on_cpu():
 
 
 def test_search_space_expansion_follows_the_reference_yaml_layout():
-    yaml = pytest.importorskip("yaml")
-    path = os.path.join(REF_PKG, "cuvs_bench", "config", "algos", "cuvs_ivf_pq.yaml")
-    if os.path.exists(path):
-        group = yaml.safe_load(open(path))["groups"]["test"]
-    else:  # the GPU box has no reference checkout: the same group, transcribed
-        group = {"build": {"nlist": [1024], "pq_dim": [16], "pq_bits": [6], "ratio": [1], "niter": [20]},
-                 "search": {"nprobe": [1, 5], "internalDistanceDtype": ["float"], "smemLutDtype": ["half"], "refine_ratio": [1]}}
+    group = _reference_interface()["cuvs_ivf_pq_test_group"]  # the `test` group of the reference's cuvs_ivf_pq.yaml
     seen = []
 
     class Recorder(OracleExactBackend):
@@ -109,36 +111,20 @@ def test_recall_definition():
 
 
 def test_plugin_is_a_backend_of_the_reference_package():
-    """With the reference's benchmark package importable, the plugin derives from ITS BenchmarkBackend, implements every abstract
-    method and registers with its registry (python/cuvs_bench/cuvs_bench/backends/registry.py)."""
-    if not os.path.isdir(REF_PKG):
-        pytest.skip("no reference checkout on this box")
-    sys.path.insert(0, REF_PKG)
-    try:
-        try:
-            base = importlib.import_module("cuvs_bench.backends.base")
-        except Exception as e:  # noqa: BLE001 - optional third-party imports of the reference package
-            pytest.skip(f"reference cuvs_bench not importable here: {e}")
-        mod = importlib.reload(bb)
-        try:
-            if not mod.HAVE_CUVS_BENCH:
-                pytest.skip("reference cuvs_bench.backends imports optional packages that are absent here")
-            assert issubclass(mod.CuvsB200Backend, base.BenchmarkBackend)
-            assert not getattr(mod.CuvsB200Backend, "__abstractmethods__", frozenset())
-            assert mod.register("cuvs_b200_test")
-            from cuvs_bench.backends.registry import get_registry
-            backend = get_registry().get_backend("cuvs_b200_test", {"name": "cuvs_ivf_pq.test"})
-            assert isinstance(backend, base.BenchmarkBackend)
-            res = mod.BuildResult(index_path="", build_time_seconds=1.0, index_size_bytes=2, algorithm="a", build_params={"nlist": 4})
-            assert res.to_json()["name"] == "a/build"
-        finally:
-            sys.path.remove(REF_PKG)
-            for name in [m for m in sys.modules if m == "cuvs_bench" or m.startswith("cuvs_bench.")]:
-                del sys.modules[name]
-            importlib.reload(bb)
-    finally:
-        if REF_PKG in sys.path:
-            sys.path.remove(REF_PKG)
+    """The plugin implements every abstract method of the reference's BenchmarkBackend (python/cuvs_bench/cuvs_bench/backends/
+    base.py) with the reference's parameters, and its result records are the reference's BuildResult / SearchResult JSON
+    records on the same values."""
+    gold = _reference_interface()
+    assert not getattr(bb.CuvsB200Backend, "__abstractmethods__", frozenset())
+    for name, params in gold["abstract_methods"].items():
+        attr = inspect.getattr_static(bb.CuvsB200Backend, name)
+        assert not getattr(attr, "__isabstractmethod__", False), name
+        if params is None:
+            assert isinstance(attr, property), name
+        else:
+            assert list(inspect.signature(attr).parameters) == params, name
+    assert bb.BuildResult(**BUILD_RESULT).to_json() == gold["build_result_json"]
+    assert bb.SearchResult(**SEARCH_RESULT).to_json() == gold["search_result_json"]
 
 
 def test_c0_through_the_reference_orchestrator(tmp_path):
@@ -220,26 +206,11 @@ def test_c0_through_the_reference_orchestrator(tmp_path):
 
 def test_recall_and_grid_expansion_agree_with_the_reference_helpers():
     """bb.recall_at_k vs cuvs_bench.backends._utils.compute_recall, and run_config's Cartesian expansion vs expand_param_grid
-    (python/cuvs_bench/cuvs_bench/backends/_utils.py:125-215), on random inputs — executed against the reference package."""
-    if not os.path.isdir(REF_PKG):
-        pytest.skip("no reference checkout on this box")
-    sys.path.insert(0, REF_PKG)
-    try:
-        try:
-            ref = importlib.import_module("cuvs_bench.backends._utils")
-        except Exception as e:  # noqa: BLE001
-            pytest.skip(f"reference helpers not importable here: {e}")
-        rng = np.random.default_rng(3)
-        for k, gtk in [(8, 16), (10, 10), (1, 5), (12, 12)]:  # set recall over the first k ground-truth ids (_utils.py:156-204)
-            found = np.stack([rng.permutation(40)[:k] for _ in range(25)])
-            truth = np.stack([rng.permutation(40)[:gtk] for _ in range(25)])
-            assert bb.recall_at_k(found, truth, k) == pytest.approx(ref.compute_recall(found, truth, k))
-        grid = {"nlist": [1024, 2048], "pq_dim": [64, 32], "ratio": [10]}
-        mine = [dict(zip(sorted(grid), vals)) for vals in __import__("itertools").product(*[grid[x] for x in sorted(grid)])]
-        theirs = ref.expand_param_grid(grid)
-        assert sorted(map(lambda d: sorted(d.items()), mine)) == sorted(map(lambda d: sorted(d.items()), theirs))
-    finally:
-        for name in [m for m in sys.modules if m == "cuvs_bench" or m.startswith("cuvs_bench.")]:
-            del sys.modules[name]
-        if REF_PKG in sys.path:
-            sys.path.remove(REF_PKG)
+    (python/cuvs_bench/cuvs_bench/backends/_utils.py:125-215), on seeded inputs — the reference's answers recorded."""
+    gold = _reference_interface()
+    for (found, truth, k), want in zip(recall_inputs(), gold["recall"], strict=True):  # set recall over the first k ids
+        assert bb.recall_at_k(found, truth, k) == pytest.approx(want)
+    grid = gold["param_grid"]
+    mine = [dict(zip(sorted(grid), vals)) for vals in itertools.product(*[grid[x] for x in sorted(grid)])]
+    theirs = gold["param_grid_expanded"]
+    assert sorted(map(lambda d: sorted(d.items()), mine)) == sorted(map(lambda d: sorted(d.items()), theirs))

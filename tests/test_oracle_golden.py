@@ -161,31 +161,15 @@ def test_oracle_knn_reproduces_the_reference_cpu_search(case):
 
 
 def test_fp8_restatement_equals_the_reference_code_compiled_here():
-    """oracle/_ref/libref_fp8.so is the REFERENCE's fp_8bit<5, Signed> (cpp/src/neighbors/ivf_pq/ivf_pq_fp_8bit.cuh:31-100)
-    compiled from the reference source where it lies (oracle/ref_fp8/Makefile; built by __graft_entry__.build() when
-    /root/reference is present).  The oracle's restatement must agree with it on every byte and on a dense sweep of floats,
+    """The REFERENCE's fp_8bit<5, Signed> (cpp/src/neighbors/ivf_pq/ivf_pq_fp_8bit.cuh:31-100), compiled from the reference
+    source by oracle/ref_fp8/Makefile, recorded every decode and a dense sweep of encodes in tests/golden/reference_fp8.npz
+    (oracle/make_golden_fp8.py).  The oracle's restatement must agree with it on every byte and on every float of the sweep,
     for both the unsigned and the signed variant."""
-    import ctypes as C
-    so = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_fp8.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref/libref_fp8.so not built (no reference checkout on this box)")
-    ref = C.CDLL(so)
-    ref.ref_fp8_encode.restype, ref.ref_fp8_encode.argtypes = C.c_uint8, [C.c_float, C.c_int]
-    ref.ref_fp8_decode.restype, ref.ref_fp8_decode.argtypes = C.c_float, [C.c_uint8, C.c_int]
-    ref.ref_fp8_decode_half.restype, ref.ref_fp8_decode_half.argtypes = C.c_float, [C.c_uint8, C.c_int]
-    rng = np.random.default_rng(0)
-    floats = np.concatenate([
-        np.array([0.0, -0.0, 1e-30, 1e-8, 2.0 ** -16, 2.0 ** -15, 2.0 ** -14, 0.5, 1.0, 1.5, 2.0, 3.999, 1000.0, 65504.0, 1e9,
-                  1e30, np.inf], np.float32),
-        (10.0 ** rng.uniform(-7, 7, 4000)).astype(np.float32),
-        rng.standard_normal(2000).astype(np.float32) * 100.0,
-        np.float32(2.0) ** np.arange(-20, 20, dtype=np.float32),
-        np.nextafter(np.float32(2.0) ** np.arange(-18, 18, dtype=np.float32), np.float32(0)),
-    ]).astype(np.float32)
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_fp8.npz"))
+    floats = gold["floats"]
     for signed in (0, 1):
         codes = np.arange(256, dtype=np.uint8)
-        dec_ref = np.array([ref.ref_fp8_decode(int(b), signed) for b in codes], np.float32)
-        dec_half = np.array([ref.ref_fp8_decode_half(int(b), signed) for b in codes], np.float32)
+        dec_ref, dec_half = gold[f"decode_{signed}"], gold[f"decode_half_{signed}"]
         np.testing.assert_array_equal(oracle.fp8_decode(codes, signed=bool(signed)), dec_ref)
         # the reference's HALF decode (fp_8bit2half, :88-99) is the same bit trick on a 5-bit fp16 exponent: it agrees with the
         # float decode wherever the value is a normal fp16 number, and differs only in the lowest exponent (codes 0..7: fp16
@@ -194,8 +178,7 @@ def test_fp8_restatement_equals_the_reference_code_compiled_here():
         assert set(np.nonzero(~(dec_half == dec_ref))[0].tolist()) <= set(range(8)) | set(range(248, 256))
         xs = floats if signed else floats[floats >= 0]
         xs = np.concatenate([xs, -xs]) if signed else xs
-        enc_ref = np.array([ref.ref_fp8_encode(float(v), signed) for v in xs], np.uint8)
-        np.testing.assert_array_equal(oracle.fp8_encode(xs, signed=bool(signed)), enc_ref)
+        np.testing.assert_array_equal(oracle.fp8_encode(xs, signed=bool(signed)), gold[f"encode_{signed}"])
     # unsigned encode of negative inputs: "all small and negative numbers are truncated to zero" (ivf_pq_fp_8bit.cuh:62-63)
     neg = -np.abs(floats[1:200])
-    np.testing.assert_array_equal(oracle.fp8_encode(neg), np.array([ref.ref_fp8_encode(float(v), 0) for v in neg], np.uint8))
+    np.testing.assert_array_equal(oracle.fp8_encode(neg), gold["encode_negative_0"])
