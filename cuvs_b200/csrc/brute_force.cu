@@ -29,7 +29,6 @@
 #include <algorithm>
 #include <cfloat>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 #include <fstream>
 #include <memory>
@@ -347,12 +346,11 @@ static void bf_search(resources* res, const bf_index& idx, const DLTensor& qt, c
   }
 
   const bool select_min = metric_is_min_close(idx.metric);
-  static const bool force_exact = getenv("CUVS_B200_FORCE_EXACT") != nullptr;  // test knob
   // k <= 24: fused lists of 16 / 32, merged to the list length.  24 < k <= 64 (the reference's fused range,
   // knn_brute_force.cuh:447-451): fused lists of 32 per (column half, split), merged to 64 / 96 candidates, and the
   // certificate additionally uses the lists' own worst entries (bf_cands::floor) — a row of the true top-k can only be missing
   // when more than 32 of them fall into one list, which the certificate detects (flagged queries take the exact path).
-  const bool use_tc     = idx.tc && filt.kind == 0 && k <= 64 && idx.n > 0 && !force_exact;
+  const bool use_tc     = idx.tc && filt.kind == 0 && k <= 64 && idx.n > 0;
   set_last_flagged(0);
   if (!use_tc) {
     search_exact(res, idx, q, nq, 0, k, out_idx, out_dist, filt);

@@ -66,8 +66,6 @@ struct cagra_index {
 
 namespace {
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
 constexpr uint32_t kInvalid = 0xffffffffu;
 constexpr uint32_t kMsb     = 0x80000000u;
 
@@ -176,7 +174,6 @@ struct cagra_launch {
   // gathers of the iteration are in flight at once, and the team loads below (2 rows per team in flight, register-bound at
   // 40 registers / 3 CTAs per SM) find them in L2 instead of paying the HBM latency 8 times in a row.
   uint32_t prefetch_row_bytes;
-  int prefetch_mode;  // 1 = per-lane prefetch.global.L2 of the row's lines, 2 = one cp.async.bulk.prefetch.L2 per row
 };
 
 // squared L2 / negative dot between the smem query and a dataset row, computed by a team of 8 lanes
@@ -405,14 +402,7 @@ __global__ void __launch_bounds__(512, (EI <= 2 ? 3 : (EI <= 4 ? 2 : 1))) cagra_
         const uint32_t id = scand[c];
         const void* row   = p.data16 ? static_cast<const void*>(p.data16 + static_cast<int64_t>(id) * p.ld16)
                                      : static_cast<const void*>(p.data + static_cast<int64_t>(id) * p.ld);
-        if (p.prefetch_mode == 2) {
-          ptx::bulk_prefetch_l2(row, p.prefetch_row_bytes);  // UBLKPF: uniform-register operands -> one trip of a lane loop per row
-        } else {
-          // per-lane line prefetches (no uniform-register round trip): every 128-byte line the row touches
-          const char* r0 = static_cast<const char*>(row);
-          const char* l0 = reinterpret_cast<const char*>(reinterpret_cast<uintptr_t>(r0) & ~uintptr_t(127));
-          for (const char* l = l0; l < r0 + p.prefetch_row_bytes; l += 128) asm volatile("prefetch.global.L2 [%0];" ::"l"(l));
-        }
+        ptx::bulk_prefetch_l2(row, p.prefetch_row_bytes);  // UBLKPF: uniform-register operands -> one trip of a lane loop per row
       }
     }
     // ---- distances: 4 candidates per step (teams of 8 lanes), two steps in flight
@@ -580,11 +570,11 @@ cagra_plan make_plan(const cuvsCagraSearchParams& sp, int64_t n, int degree, int
 }
 
 // Row bytes for the walk's bulk L2 prefetch (0 = off): rows must start on 16-byte boundaries and be a 16-byte multiple long.
-// CUVS_B200_CAGRA_PREFETCH=0 disables it (A/B).
+// Measured on a B200 (profiles/r02_ab_cagra_prefetch.txt; 10M x 96 fp32, batch 10k): no prefetch 5.73-5.75 ms, per-lane
+// prefetch.global.L2 of the row's lines 6.06-6.08 ms (slower: three CCTL per row and lane compete with the team loads for the
+// LSU), bulk prefetch 5.56-5.58 ms.
 static uint32_t walk_prefetch_bytes(const cagra_launch& p)
 {
-  const char* e = getenv("CUVS_B200_CAGRA_PREFETCH");  // (read per search: one process can A/B)
-  if (e != nullptr && e[0] == '0') return 0;
   const size_t pitch = p.data16 ? static_cast<size_t>(p.ld16) * 2 : static_cast<size_t>(p.ld) * 4;
   const uintptr_t base = p.data16 ? reinterpret_cast<uintptr_t>(p.data16) : reinterpret_cast<uintptr_t>(p.data);
   if (pitch % 16 != 0 || base % 16 != 0) return 0;
@@ -617,9 +607,6 @@ void launch_search(cudaStream_t s, const cagra_launch& p, size_t per_warp_smem)
   cagra_launch pl = p;
   pl.work_counter = counter.data();
   pl.prefetch_row_bytes = walk_prefetch_bytes(p);
-  // measured (10M x 96 fp32, batch 10k, one box, scripts/ab_cagra.py): off 5.73-5.75 ms, line prefetches 6.06-6.08 ms (slower: three
-  // CCTL per row and lane compete with the team loads for the LSU), bulk prefetch 5.56-5.58 ms -> the bulk form is the default
-  pl.prefetch_mode      = [] { const char* e = getenv("CUVS_B200_CAGRA_PREFETCH"); return e != nullptr && e[0] == '1' ? 1 : 2; }();
   timed_section ts("cagra_search", s);
   count_launch();
   kern<<<grid, warps * 32, smem, s>>>(pl);

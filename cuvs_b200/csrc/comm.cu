@@ -89,8 +89,6 @@ __global__ void unpack_parts_kernel(const uint8_t* __restrict__ in, int64_t coun
   vals[t] = reinterpret_cast<const int64_t*>(p + ((count * 4 + 7) & ~int64_t(7)))[e];
 }
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
 }  // namespace
 
 /** One NCCL communicator per participating device of THIS process (1 for the process-per-GPU mode). */

@@ -12,6 +12,7 @@
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
+#include <cstdlib>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -243,6 +244,16 @@ void widen_to_f32(struct resources* res, const DLTensor& src, f32_matrix& out);
 void dl_fill_view(DLManagedTensor* out, void* data, int device, DLDataType dt, int ndim, const int64_t* shape);
 
 inline bool metric_is_min_close(cuvsDistanceType m) { return m != InnerProduct; }
+inline bool is_l2(cuvsDistanceType m) { return m == L2Expanded || m == L2SqrtExpanded || m == L2Unexpanded || m == L2SqrtUnexpanded; }
+
+inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
+
+/** Integer value of environment variable `name`, `dflt` when it is unset. */
+inline int64_t env_int(const char* name, int64_t dflt)
+{
+  const char* v = getenv(name);
+  return v ? atoll(v) : dflt;
+}
 
 inline int sm_count_of(int device)
 {

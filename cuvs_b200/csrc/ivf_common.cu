@@ -495,8 +495,6 @@ __global__ void sum_scores_kernel(const float* __restrict__ s, const float* __re
   if ((threadIdx.x & 31) == 0) atomicAdd(out, acc);
 }
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
 }  // namespace
 
 void tc_rows::build(cudaStream_t s, const float* x, int64_t n_, int d_, const float* xn, bool with_lo, const float* row_scale)

@@ -56,10 +56,6 @@ struct ivf_flat_index {
 
 namespace {
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
-bool is_l2(cuvsDistanceType m) { return m == L2Expanded || m == L2SqrtExpanded || m == L2Unexpanded || m == L2SqrtUnexpanded; }
-
 __global__ void scatter_rows_kernel(const float* __restrict__ src, int64_t n, int d, const int64_t* __restrict__ dst_rows,
                                     const int64_t* __restrict__ src_ids, int64_t id0, float* __restrict__ dst,
                                     int64_t* __restrict__ dst_ids)
@@ -353,7 +349,7 @@ void ivf_flat_search(resources* res, const ivf_flat_index& idx, uint32_t n_probe
   const bool use_bound = KC >= k + k / 2;
   const int lists = tc_lists_per_item();
   const int KCW   = KC * lists;
-  B2_EXPECTS(KCW >= k, "ivf_flat search: k = %d needs the two-list tensor-core epilogue (CUVS_B200_TC_EPIW=8)", k);
+  B2_EXPECTS(KCW >= k, "ivf_flat search: k = %d exceeds the %d candidates kept per probe", k, KCW);
   probe_buckets pb;
   bucket_probes(res, probes.data(), nq, static_cast<int>(n_probes), idx.n_lists, idx.lists.d_offsets.data(), KCW, pb);
 

@@ -84,8 +84,6 @@ struct ivf_pq_index {
 
 namespace {
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
 void ensure_flat_codes(resources* res, const ivf_pq_index& idx)
 {
   const size_t need = static_cast<size_t>(std::max<int64_t>(idx.lists.rows_total, 1)) * idx.pq_dim;
@@ -94,7 +92,6 @@ void ensure_flat_codes(resources* res, const ivf_pq_index& idx)
   idx.codes.alloc(need);
   pq_stream_to_flat(res->stream, idx.cstream.data(), idx.lists.rows_total, idx.pq_dim, idx.codes.data());
 }
-bool is_l2(cuvsDistanceType m) { return m == L2Expanded || m == L2SqrtExpanded || m == L2Unexpanded || m == L2SqrtUnexpanded; }
 bool is_ip(cuvsDistanceType m) { return m == InnerProduct || m == CosineExpanded; }
 
 // ------------------------------------------------------------------ fp_8bit<5, Signed> (ivf_pq_fp_8bit.cuh:31-100)
@@ -593,8 +590,7 @@ void refresh_decoded(resources* res, ivf_pq_index& idx)
   idx.cstream.release();
   idx.cb_words.release();
   if (idx.conservative || !tc_supported(res->device, idx.rot_dim)) { idx.yhat.release(); idx.hx.release(); return; }
-  static const bool keep_decoded = getenv("CUVS_B200_PQ_KEEP_DECODED") != nullptr;  // A/B experiments against path (B)
-  if (!keep_decoded && idx.Kp == idx.rot_dim &&
+  if (idx.Kp == idx.rot_dim &&
       pq_stream_supported(res->device, idx.pq_dim, idx.pq_len, idx.pq_bits, idx.codebook_kind == CUVS_IVF_PQ_CODEBOOK_GEN_PER_SUBSPACE)) {
     idx.cstream.alloc(static_cast<size_t>(std::max<int64_t>(R / 128, 1)) * pq_stream_tile_bytes(idx.pq_dim));
     idx.cb_words.alloc(static_cast<size_t>(idx.pq_dim / 32) * 256 * 32);
@@ -604,8 +600,7 @@ void refresh_decoded(resources* res, ivf_pq_index& idx)
     // hundreds of queries to every list (10M vectors / 1024 lists / 10k x 64 probes = 625 per list) the stream kernel would
     // decode each list once per 64 probing queries, and reading rows decoded once at build time is the better trade.  The
     // search picks per call (dense_probing below).  Budget: CUVS_B200_PQ_DECODED_BUDGET_MB (default 4096, 0 = never).
-    const char* bm        = getenv("CUVS_B200_PQ_DECODED_BUDGET_MB");
-    const int64_t budget  = (bm ? atoll(bm) : 4096) << 20;
+    const int64_t budget  = env_int("CUVS_B200_PQ_DECODED_BUDGET_MB", 4096) << 20;
     const bool also_rows  = R > 0 && static_cast<int64_t>(R) * idx.Kp * 2 <= budget;
     if (also_rows) {
       idx.yhat.alloc(static_cast<size_t>(std::max<int64_t>(R, 128)) * idx.Kp);
@@ -622,8 +617,7 @@ void refresh_decoded(resources* res, ivf_pq_index& idx)
       idx.yhat.release();
       idx.hx.release();
     }
-    static const bool keep_flat = getenv("CUVS_B200_PQ_KEEP_FLAT") != nullptr;
-    if (!keep_flat && R > 0) {  // the stream is the index: pq_dim + 4 bytes per vector (+ 8 for the id)
+    if (R > 0) {  // the stream is the index: pq_dim + 4 bytes per vector (+ 8 for the id)
       B2_CUDA(cudaStreamSynchronize(s));
       idx.codes.release();
     }
@@ -910,7 +904,7 @@ void ivf_pq_search(resources* res, const ivf_pq_index& idx, const cuvsIvfPqSearc
   // them fall into one half — an approximation only the k > 32 candidate-generation use case can see)
   const int KC    = k <= 16 ? 16 : (k <= 32 || (use_tc && !use_stream) ? 32 : 64);
   const int KCW   = KC * lists;
-  B2_EXPECTS(KCW >= k, "ivf_pq search: k = %d > 64 needs an index with decoded rows (CUVS_B200_PQ_KEEP_DECODED=1) or the LUT path (CUVS_B200_PQ_PATH=lut)", k);
+  B2_EXPECTS(KCW >= k, "ivf_pq search: k = %d exceeds the %d candidates kept per probe", k, KCW);
   // queries per work item: 128 for the query-major kernels; the streamed kernel takes the list rows as the MMA's M side
   // and 32 / 64 / 128 probing queries as N (picked from the average number of pairs per list)
   const int group = use_stream ? pq_stream_group(static_cast<double>(nq) * n_probes / std::max<uint32_t>(idx.n_lists, 1), KC, passes) : 128;
@@ -987,23 +981,6 @@ void ivf_pq_search(resources* res, const ivf_pq_index& idx, const cuvsIvfPqSearc
     B2_CUDA(cudaGetLastError());
   }
 
-  if (const char* dump = getenv("CUVS_B200_PQ_DUMP")) {
-    // debug: raw per-(query, probe) candidate lists of the fine scan -> file (slot_of [nq*n_probes] u32, cs / cp [n_pairs*KCW])
-    B2_CUDA(cudaStreamSynchronize(s));
-    std::vector<uint32_t> h_slot(static_cast<size_t>(nq) * n_probes), h_cp(static_cast<size_t>(pb.n_pairs) * KCW), h_probes(static_cast<size_t>(nq) * n_probes);
-    std::vector<float> h_cs(static_cast<size_t>(pb.n_pairs) * KCW);
-    B2_CUDA(cudaMemcpy(h_slot.data(), pb.slot_of.data(), h_slot.size() * 4, cudaMemcpyDeviceToHost));
-    B2_CUDA(cudaMemcpy(h_probes.data(), probes.data(), h_probes.size() * 4, cudaMemcpyDeviceToHost));
-    B2_CUDA(cudaMemcpy(h_cp.data(), cp.data(), h_cp.size() * 4, cudaMemcpyDeviceToHost));
-    B2_CUDA(cudaMemcpy(h_cs.data(), cs.data(), h_cs.size() * 4, cudaMemcpyDeviceToHost));
-    std::ofstream os(dump, std::ios::binary);
-    const int64_t hdr[4] = {nq, static_cast<int64_t>(n_probes), KCW, pb.n_pairs};
-    os.write(reinterpret_cast<const char*>(hdr), sizeof(hdr));
-    os.write(reinterpret_cast<const char*>(h_slot.data()), h_slot.size() * 4);
-    os.write(reinterpret_cast<const char*>(h_probes.data()), h_probes.size() * 4);
-    os.write(reinterpret_cast<const char*>(h_cs.data()), h_cs.size() * 4);
-    os.write(reinterpret_cast<const char*>(h_cp.data()), h_cp.size() * 4);
-  }
   // ---- per query: concatenate its probes' candidates (already in final distance units), top-k, ids
   const int64_t cand_w = static_cast<int64_t>(n_probes) * KCW;
   dbuf<uint32_t> mp(static_cast<size_t>(nq) * k, s);

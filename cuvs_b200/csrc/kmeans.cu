@@ -23,8 +23,6 @@
 namespace b200 {
 namespace {
 
-inline unsigned blocks_for(int64_t n, int bs) { return static_cast<unsigned>((n + bs - 1) / bs); }
-
 __global__ void u32_to_i32_kernel(const uint32_t* in, int32_t* out, int64_t n)
 {
   int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;

@@ -82,12 +82,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
     ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
     : "memory");
 }
-// 2-D tile prefetch into L2 (no shared-memory destination, no barrier)
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* m, int32_t c0, int32_t c1)
-{
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(m)), "r"(c0), "r"(c1)
-               : "memory");
-}
 // 1-D bulk copy global -> shared (16-byte aligned, size multiple of 16)
 __device__ __forceinline__ void bulk_load_1d(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar)
 {
@@ -120,20 +114,9 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr)
 __device__ __forceinline__ void tc_fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem] * B[smem], bf16 inputs, fp32 accumulate, issued by ONE thread
-__device__ __forceinline__ void mma_bf16_ss(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
-{
-  asm volatile(
-    "{\n\t"
-    ".reg .pred p;\n\t"
-    "setp.ne.b32 p, %4, 0;\n\t"
-    "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %6, %7, %8}, p;\n\t"
-    "}\n"
-    ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate), "r"(0u), "r"(0u), "r"(0u), "r"(0u)
-    : "memory");
-}
-// Same, with the two shared-memory descriptors given as (lo, hi) 32-bit halves: consecutive K steps / stages differ only
-// in the low word (start address >> 4), so the issuing thread spends one integer add per operand and MMA.
+// D[tmem] (+)= A[smem] * B[smem], bf16 inputs, fp32 accumulate, issued by ONE thread.  The two shared-memory descriptors are
+// given as (lo, hi) 32-bit halves: consecutive K steps / stages differ only in the low word (start address >> 4), so the
+// issuing thread spends one integer add per operand and MMA.
 __device__ __forceinline__ void mma_bf16_ss_lohi(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi,
                                                  uint32_t idesc, uint32_t accumulate)
 {
@@ -172,17 +155,6 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32])
     : "r"(taddr)
     : "memory");
 }
-// 16-column variant
-__device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&r)[16])
-{
-  asm volatile(
-    "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-    "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-    : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-      "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-    : "r"(taddr)
-    : "memory");
-}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads)
@@ -190,28 +162,6 @@ __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads)
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
 
-// K-major operand tile in shared memory, 128-byte swizzle: rows of 128 bytes, 8-row groups 1024 B apart.
-__device__ __forceinline__ uint64_t make_smem_desc_sw128(uint32_t smem_addr)
-{
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3ffffu) >> 4);  // start address, 16-byte units
-  d |= static_cast<uint64_t>(1) << 16;                      // leading byte offset (unused for swizzled K-major)
-  d |= static_cast<uint64_t>(1024 >> 4) << 32;              // stride byte offset between 8-row groups
-  d |= static_cast<uint64_t>(1) << 46;                      // descriptor version (Blackwell)
-  d |= static_cast<uint64_t>(2) << 61;                      // SWIZZLE_128B
-  return d;
-}
-// K-major operand tile, 32-byte swizzle: rows of 32 bytes (one K=16 bf16 step), 8-row groups 256 B apart.
-__device__ __forceinline__ uint64_t make_smem_desc_sw32(uint32_t smem_addr)
-{
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr & 0x3ffffu) >> 4);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(256 >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(6) << 61;  // SWIZZLE_32B
-  return d;
-}
 // kind::f16, A = B = bf16, D = fp32, both K-major, dense
 __host__ __device__ constexpr uint32_t make_idesc_bf16(int M, int N)
 {

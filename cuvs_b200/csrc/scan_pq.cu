@@ -30,24 +30,15 @@
 #include "timing.hpp"
 
 #include <cuda.h>
-#include <unistd.h>
 
 #include <cmath>
-#include <cstdio>
-#include <cstdlib>
-#include <cstring>
 #include <mutex>
 
 namespace b200 {
 namespace {
 
 constexpr int kDecWarps   = 8;
-#ifndef CUVS_B200_PQ_EPI_WARPS
-#define CUVS_B200_PQ_EPI_WARPS 8
-#endif
-constexpr int kEpiWarps   = CUVS_B200_PQ_EPI_WARPS;  // kEpiPerQ per TMEM lane quarter: they split the (tile, chunk) units of a round
-constexpr int kEpiPerQ    = kEpiWarps / 4;
-static_assert(kEpiWarps % 4 == 0 && kEpiPerQ >= 2 && kEpiPerQ <= 4, "epilogue warps come in groups of four (one per lane quarter)");
+constexpr int kEpiWarps   = 8;  // two per TMEM lane quarter: they split the (tile, chunk) units of a round
 constexpr int kEpiThreads = 32 * kEpiWarps;
 constexpr int kThreads    = 64 + 32 * kDecWarps + kEpiThreads;  // 576
 constexpr int kEpiWarp0   = 2 + kDecWarps;                      // first epilogue warp (10: warp & 3 covers all TMEM quarters)
@@ -78,43 +69,7 @@ struct pq_args {
   int cap;      // candidate buffer entries per query (KC < cap <= 128)
   int cstages;  // code ring depth
   int blk;      // bytes of one tile block of the stream
-  int tb_limit;   // tiles per epilogue round (<= layout::tb; CUVS_B200_PQ_TB for bisection)
-  int dbg_mode;   // CUVS_B200_PQ_DEBUG value: 2 = the epilogue only drains TMEM (no filtering): pipeline-only bisection
-  uint32_t* dbg;  // CUVS_B200_PQ_DEBUG=1: mapped host memory, [grid][8] = {code of the wait that timed out, parity, item, tile, ...}
 };
-
-// Debug wait: identical to ptx::mbar_wait unless P.dbg is set; then a wait that does not complete within ~2 s records where
-// it is stuck (role/barrier code, parity, progress counters) in mapped host memory and traps, so a deadlock becomes a report.
-// (Out of line: the kernel has ~15 wait sites and its instruction footprint matters — see the i-cache note at do_chunk.)
-__device__ __noinline__ void wait_dbg_slow(uint32_t* dbg, uint64_t* bar, uint32_t parity, uint32_t code, uint32_t a, uint32_t b)
-{
-  for (uint32_t spin = 0; spin < 4000000u; ++spin) {
-    uint32_t ok;
-    asm volatile(
-      "{\n\t"
-      ".reg .pred P;\n\t"
-      "mbarrier.test_wait.parity.shared::cta.b64 P, [%1], %2;\n\t"
-      "selp.b32 %0, 1, 0, P;\n\t"
-      "}\n"
-      : "=r"(ok)
-      : "r"(ptx::smem_u32(bar)), "r"(parity)
-      : "memory");
-    if (ok) return;
-    __nanosleep(500);
-  }
-  if ((threadIdx.x & 31) == 0) {
-    uint32_t* d = dbg + blockIdx.x * 16;
-    if (atomicCAS(d, 0u, code) == 0u) { d[1] = parity; d[2] = a; d[3] = b; d[4] = threadIdx.x >> 5; }
-    __threadfence_system();
-  }
-  __nanosleep(100000000);
-  __trap();
-}
-__device__ __forceinline__ void wait_dbg(uint32_t* dbg, uint64_t* bar, uint32_t parity, uint32_t code, uint32_t a, uint32_t b)
-{
-  if (dbg == nullptr) ptx::mbar_wait(bar, parity);
-  else wait_dbg_slow(dbg, bar, parity, code, a, b);
-}
 
 __device__ __forceinline__ bool bar_red_or(uint32_t id, uint32_t nthreads, bool pred)
 {
@@ -381,7 +336,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
     // ------------------------------------------------------------------ producer (whole warp loops, one elected lane issues)
     uint32_t cs = 0, cph = 0, qph = 0, ss = 0, sp = 0;
     for (;;) {
-      wait_dbg(P.dbg, &s_empty[ss], sp ^ 1, 0x101, ss, 0);
+      ptx::mbar_wait(&s_empty[ss], sp ^ 1);
       int it = 0;
       if (lane == 0) {
         it = atomicAdd(P.sched, 1);
@@ -396,7 +351,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
       item.a_row0  = __shfl_sync(0xffffffffu, item.a_row0, 0);
       item.b_row0  = __shfl_sync(0xffffffffu, item.b_row0, 0);
       item.n_tiles = __shfl_sync(0xffffffffu, item.n_tiles, 0);
-      wait_dbg(P.dbg, q_empty, qph ^ 1, 0x102, static_cast<uint32_t>(it), 0);
+      ptx::mbar_wait(q_empty, qph ^ 1);
       if (ptx::elect_one()) {
         ptx::mbar_arrive_expect_tx(q_full, L::q_bytes);
 #pragma unroll
@@ -408,7 +363,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
       qph ^= 1;
       const uint8_t* src = P.stream + static_cast<int64_t>(item.b_row0 >> 7) * P.blk;
       for (uint32_t t = 0; t < item.n_tiles; ++t) {
-        wait_dbg(P.dbg, &c_empty[cs], cph ^ 1, 0x103, static_cast<uint32_t>(it), t);
+        ptx::mbar_wait(&c_empty[cs], cph ^ 1);
         if (ptx::elect_one()) {
           ptx::mbar_arrive_expect_tx(&c_full[cs], static_cast<uint32_t>(P.blk));
           ptx::bulk_load_1d(sCode + cs * P.blk, src + static_cast<int64_t>(t) * P.blk, static_cast<uint32_t>(P.blk), &c_full[cs]);
@@ -423,7 +378,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
     const uint32_t ones_lo = ptx::smem_desc_lo(ptx::smem_u32(sOnes));
     uint32_t ds = 0, dph = 0, acc = 0, aph = 0, qph = 0, ss = 0, sp = 0;
     for (;;) {
-      wait_dbg(P.dbg, &s_full[ss], sp, 0x201, ss, 0);
+      ptx::mbar_wait(&s_full[ss], sp);
       const int it = __shfl_sync(0xffffffffu, s_item[ss], 0);  // (the shuffle consumes the load before the slot is handed back)
       if (lane == 0) ptx::mbar_arrive(&s_empty[ss]);
       if (++ss == kSched) { ss = 0; sp ^= 1; }
@@ -432,11 +387,11 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
       // N of the MMA = the item's live queries rounded up to 16: a narrow item neither reads nor multiplies the unused rows
       const uint32_t n_live = min(static_cast<uint32_t>(NQ), (__shfl_sync(0xffffffffu, P.items[it].valid_rows, 0) + 15u) & ~15u);
       const uint32_t idesc  = ptx::make_idesc_bf16(128, static_cast<int>(max(n_live, 16u)));
-      wait_dbg(P.dbg, q_full, qph, 0x202, static_cast<uint32_t>(it), 0);
+      ptx::mbar_wait(q_full, qph);
       ptx::tc_fence_after_sync();
       for (uint32_t t = 0; t < n_tiles; ++t) {
-        wait_dbg(P.dbg, &t_empty[acc], aph ^ 1, 0x203, static_cast<uint32_t>(it), t);
-        wait_dbg(P.dbg, &d_full[ds], dph, 0x204, static_cast<uint32_t>(it), t);
+        ptx::mbar_wait(&t_empty[acc], aph ^ 1);
+        ptx::mbar_wait(&d_full[ds], dph);
         ptx::tc_fence_after_sync();
         if (ptx::elect_one()) {
           const uint32_t d_tmem = tmem_base + acc * NQ;
@@ -475,14 +430,14 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
     const uint32_t cb_lane32 = ptx::smem_u32(sCb) + static_cast<uint32_t>(lane) * 4u;  // this lane's word of codebook row 0
     uint32_t cs = 0, cph = 0, ds = 0, dph = 0, ss = 0, sp = 0;
     for (;;) {
-      wait_dbg(P.dbg, &s_full[ss], sp, 0x301, ss, 0);
+      ptx::mbar_wait(&s_full[ss], sp);
       const int it = __shfl_sync(0xffffffffu, s_item[ss], 0);  // (consumes the load before the slot is handed back)
       if (lane == 0) ptx::mbar_arrive(&s_empty[ss]);
       if (++ss == kSched) { ss = 0; sp ^= 1; }
       if (it < 0) break;
       const uint32_t n_tiles = P.items[it].n_tiles;
       for (uint32_t t = 0; t < n_tiles; ++t) {
-        wait_dbg(P.dbg, &c_full[cs], cph, 0x302, static_cast<uint32_t>(it), t);
+        ptx::mbar_wait(&c_full[cs], cph);
         const uint8_t* cst = sCode + cs * P.blk;
         uint4 cw[NKB];
 #pragma unroll
@@ -497,7 +452,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
         const uint32_t cs_read = cs;
         if (++cs == ncs) { cs = 0; cph ^= 1; }
 
-        wait_dbg(P.dbg, &d_empty[ds], dph ^ 1, 0x303, static_cast<uint32_t>(it), t);
+        ptx::mbar_wait(&d_empty[ds], dph ^ 1);
         uint8_t* dst = sDec + ds * L::dec_stage + (2 * dw) * 1024;
 #pragma unroll
         for (int h = 0; h < NKB; ++h) {
@@ -544,7 +499,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
     // ------------------------------------------------------------------ epilogue: thread = list row, columns = queries
     const int ew      = warp - kEpiWarp0;
     const int quarter = warp & 3;
-    const int half    = ew >> 2;  // which of the lane quarter's kEpiPerQ warps: they split the round's (tile, chunk) units
+    const int half    = ew >> 2;  // which of the lane quarter's two warps: they split the round's (tile, chunk) units
     const int row     = quarter * 32 + lane;
     const int te      = static_cast<int>(threadIdx.x) - 32 * kEpiWarp0;  // 0..127
     const uint32_t t_lane = tmem_base + (static_cast<uint32_t>(quarter * 32) << 16);
@@ -573,18 +528,9 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
       if (lane == 0) sCnt[col] = min(n, KC);
       __syncwarp();
     };
-
-    auto mark = [&](uint32_t stage) {  // epilogue progress markers for the deadlock report (compiled in with -DCUVS_B200_PQ_MARKS)
-#ifdef CUVS_B200_PQ_MARKS
-      if (P.dbg != nullptr && lane == 0) { reinterpret_cast<volatile uint32_t*>(P.dbg)[blockIdx.x * 16 + 8 + ew] = stage; __threadfence_system(); }
-#else
-      (void)stage;
-#endif
-    };
     for (;;) {
-      wait_dbg(P.dbg, &s_full[ss], sp, 0x401, ss, 0);
+      ptx::mbar_wait(&s_full[ss], sp);
       const int it = __shfl_sync(0xffffffffu, s_item[ss], 0);  // (consumes the load before the slot is handed back)
-      mark(1);
       if (lane == 0) ptx::mbar_arrive(&s_empty[ss]);
       if (++ss == kSched) { ss = 0; sp ^= 1; }
       if (it < 0) break;
@@ -604,9 +550,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
         sThr[col] = thr;
         sCnt[col] = 0;
       }
-      mark(2);
       ptx::named_bar_sync(1, kEpiThreads);
-      mark(3);
 
       auto do_chunk = [&](uint32_t taddr, uint32_t pos, int c, uint32_t only) -> uint32_t {
         return pq_filter_chunk(taddr + c * 32, pos, sThr + c * 32, sCnt + c * 32, sCand + c * 32 * cap, cap, only);
@@ -619,8 +563,8 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
       // sending one of them through 32 columns of +inf thresholds.
       const int nvc = min(NCH, (static_cast<int>(item.valid_rows) + 31) >> 5);
       // rounds of TB tiles: all their accumulators are filtered, then ONE barrier decides whether any buffer overflowed
-      for (uint32_t t0 = 0; t0 < item.n_tiles; t0 += min(TB, P.tb_limit)) {
-        const int nb = static_cast<int>(min(static_cast<uint32_t>(min(TB, P.tb_limit)), item.n_tiles - t0));
+      for (uint32_t t0 = 0; t0 < item.n_tiles; t0 += TB) {
+        const int nb = static_cast<int>(min(static_cast<uint32_t>(TB), item.n_tiles - t0));
         uint4 pend[NCH];  // per chunk: .x/.y/.z/.w = columns still pending in tile 0..3 of the round
         bool any_left = false;
 #pragma unroll
@@ -629,15 +573,7 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
 #pragma unroll 1  // ONE inlined copy of the round filter (its call overhead was ~15 % of the epilogue's instructions)
         for (int c = 0; c < nvc; ++c) {
           // tiles of the round whose (tile, c) unit is this warp's: all or none for an even chunk count, every other one else
-          uint32_t mask;
-          if (kEpiPerQ == 2) {
-            mask = live & ((nvc & 1) ? (0x55555555u << ((t0 + c + half) & 1u)) : ((c & 1) == half ? 0xffffffffu : 0u));
-          } else {  // unit (t, c) -> warp ((t * nvc + c) mod kEpiPerQ) of the quarter
-            mask = 0u;
-#pragma unroll
-            for (int b = 0; b < TB; ++b)
-              if (b < nb && static_cast<int>(((t0 + b) * nvc + c) % kEpiPerQ) == half) mask |= 1u << b;
-          }
+          const uint32_t mask = live & ((nvc & 1) ? (0x55555555u << ((t0 + c + half) & 1u)) : ((c & 1) == half ? 0xffffffffu : 0u));
           if (mask != 0u) {  // (warp-uniform)
             pend[c] = pq_filter_round(t_lane + c * 32, acc, L::acc, NQ, mask, item.b_row0 + t0 * 128 + row, sThr + c * 32, sCnt + c * 32,
                                       sCand + c * 32 * cap, cap, t_full, aph);
@@ -664,7 +600,6 @@ pq_stream_scan_kernel(const __grid_constant__ CUtensorMap tmQ_hi, const __grid_c
           }
           __syncwarp();
         }
-        mark(0x16 + (t0 << 8));
         ptx::tc_fence_before_sync();
         __syncwarp();
         if (lane == 0) {
@@ -805,64 +740,22 @@ CUtensorMap make_query_map(const __nv_bfloat16* ptr, int64_t rows, int Kp, int g
   return m;
 }
 
-int env_int(const char* name, int dflt)
-{
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 template <int NQ, int NKB, int PASSES>
 void launch(cudaStream_t stream, int sms, const CUtensorMap& mq_hi, const CUtensorMap& mq_lo, pq_args a, int n_items)
 {
   using L   = layout<NQ, NKB, PASSES>;
   auto kern = pq_stream_scan_kernel<NQ, NKB, PASSES>;
   a.cap     = a.KC <= 16 ? (NQ == 128 ? 32 : 64) : (a.KC <= 32 ? 64 : 128);  // free slots between compactions: cap - KC
-  if (const int cap_env = env_int("CUVS_B200_PQ_CAP", 0)) a.cap = std::max(a.KC + 8, std::min(128, cap_env));  // bisection knob
   const int fixed = L::off_cand + NQ * a.cap * 8 + 1024 /*alignment slack of the dynamic segment*/;
   a.cstages = std::min(kMaxCStages, (kSmemLimit - fixed) / a.blk);
-  a.tb_limit = std::max(1, std::min(L::tb, env_int("CUVS_B200_PQ_TB", L::tb)));
-  const int forced = env_int("CUVS_B200_PQ_CSTAGES", 0);  // limiter experiments only
-  if (forced > 0) a.cstages = std::min(a.cstages, forced);
   B2_EXPECTS(a.cstages >= 2, "pq_stream_scan: shared memory budget exceeded (NQ=%d KC=%d passes=%d)", NQ, a.KC, PASSES);
   const size_t smem = static_cast<size_t>(fixed) + static_cast<size_t>(a.cstages) * a.blk;
-  static uint32_t* dbg_host = nullptr;  // CUVS_B200_PQ_DEBUG=1: deadlock report (see wait_dbg)
-  if (env_int("CUVS_B200_PQ_DEBUG", 0)) {
-    if (!dbg_host) B2_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&dbg_host), 16 * sizeof(uint32_t) * 1024, cudaHostAllocMapped));
-    memset(dbg_host, 0, 16 * sizeof(uint32_t) * 1024);
-    uint32_t* dptr = nullptr;
-    B2_CUDA(cudaHostGetDevicePointer(reinterpret_cast<void**>(&dptr), dbg_host, 0));
-    a.dbg = dptr;
-    a.dbg_mode = env_int("CUVS_B200_PQ_DEBUG", 0);
-    fprintf(stderr, "[pq_stream_scan] NQ=%d NKB=%d PASSES=%d KC=%d cap=%d cstages=%d blk=%d smem=%zu items<=%d\n", NQ, NKB, PASSES, a.KC, a.cap,
-            a.cstages, a.blk, smem, n_items);
-  }
   B2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   const int grid = n_items < sms ? n_items : sms;
   timed_section ts("pq_stream_scan", stream);
   count_launch();
   kern<<<grid, kThreads, smem, stream>>>(mq_hi, mq_lo, a);
   B2_CUDA(cudaGetLastError());
-  if (a.dbg != nullptr) {
-    cudaError_t e = cudaErrorNotReady;
-    for (int i = 0; i < 80 && e == cudaErrorNotReady; ++i) {  // poll for ~8 s: a hang must not block the host forever
-      e = cudaStreamQuery(stream);
-      if (e == cudaErrorNotReady) usleep(100000);
-    }
-    int shown = 0;
-    for (int b = 0; b < grid && b < 1024 && shown < 6; ++b)
-      if (dbg_host[b * 16] || e != cudaSuccess) {
-        ++shown;
-        fprintf(stderr, "[pq_stream_scan] CTA %d: stuck wait 0x%x parity %u a=%u b=%u warp %u | epilogue stages %x %x %x %x\n", b, dbg_host[b * 16],
-                dbg_host[b * 16 + 1], dbg_host[b * 16 + 2], dbg_host[b * 16 + 3], dbg_host[b * 16 + 4], dbg_host[b * 16 + 8], dbg_host[b * 16 + 9],
-                dbg_host[b * 16 + 10], dbg_host[b * 16 + 11]);
-      }
-    if (e == cudaErrorNotReady) {
-      fprintf(stderr, "[pq_stream_scan] kernel still running after 8 s: giving up (process exits)\n");
-      fflush(stderr);
-      _exit(3);
-    }
-    B2_EXPECTS(e == cudaSuccess, "pq_stream_scan (debug): kernel failed: %s", cudaGetErrorString(e));
-  }
 }
 
 }  // namespace
@@ -899,7 +792,7 @@ void pq_stream_to_flat(cudaStream_t s, const uint8_t* stream, int64_t rows_total
 
 int pq_stream_group(double pairs_per_list, int KC, int passes)
 {
-  const int forced = env_int("CUVS_B200_PQ_GROUP", 0);  // tests and limiter experiments (read per call)
+  const int64_t forced = env_int("CUVS_B200_PQ_GROUP", 0);  // tests pin the group (read per call)
   int g = pairs_per_list <= 20.0 ? 32 : (pairs_per_list <= 80.0 ? 64 : 128);
   if (forced == 32 || forced == 64 || forced == 128) g = forced;
   if ((KC > 16 || passes == 2) && g > 64) g = 64;  // shared-memory budget: wide candidate buffers / two residual planes
@@ -926,7 +819,7 @@ void pq_stream_scan(cudaStream_t stream, int device, const __nv_bfloat16* q_hi, 
   a.out_score = out_score;
   a.out_pos = out_pos;
   a.out_row_stride = out_row_stride;
-  if (bound != nullptr && bound->keys != nullptr && !env_int("CUVS_B200_PQ_NO_BOUND", 0)) {
+  if (bound != nullptr && bound->keys != nullptr) {
     a.b_keys = bound->keys;
     a.b_idx = bound->idx;
     a.b_add = bound->add;

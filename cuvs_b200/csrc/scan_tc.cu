@@ -28,7 +28,6 @@
 #include <cuda.h>
 
 #include <cmath>
-#include <cstdlib>
 #include <mutex>
 
 namespace b200 {
@@ -41,7 +40,6 @@ constexpr int kAccBufs    = 4;          // TMEM accumulator ring
 constexpr int kEpiWarps   = 8;
 constexpr int kEpiThreads = 32 * kEpiWarps;
 constexpr int kCols       = 64;         // accumulator columns per epilogue thread and tile
-constexpr int kPrefetch   = 8;          // L2 prefetch distance of the B stream, in tiles
 constexpr int kSched      = 4;          // depth of the work-item ring between the producer and its consumers
 
 // PASSES: 1 = hi*hi; 2 = (hi + lo)*hi (exact A side: query rows at fp32 grade against bf16-exact B rows);
@@ -74,11 +72,8 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
                const __grid_constant__ CUtensorMap tmB_hi, const __grid_constant__ CUtensorMap tmB_lo,
                const __grid_constant__ CUtensorMap tmB_x, const tc_item* __restrict__ items, int n_items_host,
                const int* __restrict__ n_items_dev, int kblocks_rt, int* __restrict__ sched_counter, float* __restrict__ out_score, uint32_t* __restrict__ out_pos,
-               int64_t out_row_stride, int dbg_flags, tc_bound bound)
+               int64_t out_row_stride, tc_bound bound)
 {
-  const int dbg_skip_epilogue = dbg_flags & 1;
-  const bool prefetch_on      = (dbg_flags & 2) == 0;
-  const uint32_t nst          = (dbg_flags >> 8) ? min(static_cast<uint32_t>(dbg_flags >> 8), static_cast<uint32_t>(cfg<KB, PASSES>::stages)) : cfg<KB, PASSES>::stages;  // ring depth (experiment knob)
   using C = cfg<KB, PASSES>;
   constexpr int NA = C::NA, NB = C::NB;
   const int nkb = C::streamed ? kblocks_rt : KB;  // k-blocks of 64 per tile
@@ -186,15 +181,6 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
       }
       for (uint32_t t = 0; t < item.n_tiles; ++t) {
         const int32_t brow = static_cast<int32_t>(item.b_row0 + t * 128);
-        if (prefetch_on && lane == 0 && t + kPrefetch < item.n_tiles) {
-          const int32_t prow = brow + kPrefetch * 128;
-#pragma unroll
-          for (int kb = 0; kb < nkb; ++kb) {
-            ptx::tma_prefetch_2d(&tmB_hi, kb * 64, prow);
-            if (NB == 2) ptx::tma_prefetch_2d(&tmB_lo, kb * 64, prow);
-          }
-          ptx::tma_prefetch_2d(&tmB_x, 0, prow);
-        }
 #pragma unroll
         for (int kb = 0; kb < nkb; ++kb) {
           ptx::mbar_wait(&empty[stage], phase ^ 1);
@@ -209,7 +195,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
             if (NB == 2) ptx::tma_load_2d(dst + C::b_off + kTileBytes, &tmB_lo, &full[stage], kb * 64, brow);
             if (kb == 0) ptx::tma_load_2d(dst + C::x_off, &tmB_x, &full[stage], 0, brow);
           }
-          if (++stage == nst) { stage = 0; phase ^= 1; }
+          if (++stage == C::stages) { stage = 0; phase ^= 1; }
         }
       }
     }
@@ -262,7 +248,7 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
             ptx::mma_commit(&empty[stage]);  // frees the B stage once these MMAs have read it
           }
           b_lo += C::stage_bytes >> 4;
-          if (++stage == nst) { stage = 0; phase ^= 1; b_lo = b_lo0; }
+          if (++stage == C::stages) { stage = 0; phase ^= 1; b_lo = b_lo0; }
         }
         if (ptx::elect_one()) ptx::mma_commit(&tfull[acc]);  // accumulator complete -> epilogue
         if (++acc == kAccBufs) { acc = 0; acc_phase ^= 1; }
@@ -412,11 +398,9 @@ tc_scan_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant
         for (uint32_t t = 0; t < item.n_tiles; ++t) {
           uint32_t v0[32], v1[32];
           fetch_tile(v0, v1);
-          if (!dbg_skip_epilogue) {
-            const uint32_t pos0 = item.b_row0 + t * 128 + col0;
-            scan32(v0, pos0);
-            scan32(v1, pos0 + 32);
-          }
+          const uint32_t pos0 = item.b_row0 + t * 128 + col0;
+          scan32(v0, pos0);
+          scan32(v1, pos0 + 32);
         }
         flush();
         const float my_kth = kth_best();
@@ -489,12 +473,6 @@ CUtensorMap make_ext_map(const __nv_bfloat16* ptr, int64_t rows)
   return m;
 }
 
-int env_int(const char* name, int dflt)
-{
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 template <int KB, int PASSES, int KC>
 void launch(cudaStream_t stream, int sm_count, const CUtensorMap& a_hi, const CUtensorMap& a_lo, const CUtensorMap& b_hi,
             const CUtensorMap& b_lo, const CUtensorMap& b_x, const tc_item* items, int n_items, const int* n_items_dev,
@@ -503,11 +481,6 @@ void launch(cudaStream_t stream, int sm_count, const CUtensorMap& a_hi, const CU
   auto kern = tc_scan_kernel<KB, PASSES, KC>;
   using C   = cfg<KB, PASSES>;
   static_assert(C::smem <= 227 * 1024, "tc_scan_kernel: shared memory budget exceeded");
-  // profiling knob: MMA/TMA pipeline only (results are garbage); only honoured inside a timed region (cuvsB200TimingEnable)
-  static const int skip_env = env_int("CUVS_B200_TC_SKIP_EPI", 0);
-  static const int no_pf    = env_int("CUVS_B200_TC_PREFETCH", 0) ? 0 : 1;  // L2 prefetch of the B stream: measured no gain, off
-  // bit 0: skip the top-k work; bits 8..11: smem ring depth override (both only for the limiter experiments of profiles/README.md)
-  const int skip_epi        = (skip_env && timing_enabled() ? (skip_env & 0xf01) : 0) | (no_pf ? 2 : 0);
   // per launch, not once: the attribute belongs to the current device's context, and one process may drive several GPUs
   // (cuvsMultiGpu*); the call costs about a microsecond
   B2_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(C::smem)));
@@ -520,7 +493,7 @@ void launch(cudaStream_t stream, int sm_count, const CUtensorMap& a_hi, const CU
   timed_section ts("tc_scan", stream);
   count_launch();
   kern<<<grid, C::threads, C::smem, stream>>>(a_hi, a_lo, b_hi, b_lo, b_x, items, n_items, n_items_dev, kblocks, sched.data(), out_score,
-                                               out_pos, out_row_stride, skip_epi, bound);
+                                               out_pos, out_row_stride, bound);
   B2_CUDA(cudaGetLastError());
 }
 
@@ -638,9 +611,7 @@ void tc_scan_topk(cudaStream_t stream, int device, const __nv_bfloat16* a_hi, co
   B2_EXPECTS(passes == 1 || a_lo, "tc_scan_topk: the A lo plane is required for 2- and 3-pass mode");
   B2_EXPECTS(passes != 3 || b_lo, "tc_scan_topk: the B lo plane is required for 3-pass mode");
   const int sms = sm_count_of(device);
-  static const int no_bound = env_int("CUVS_B200_TC_NO_BOUND", 0);  // profiling knob
-  tc_bound bnd = bound ? *bound : tc_bound{};
-  if (no_bound) { bnd.keys = nullptr; }
+  const tc_bound bnd = bound ? *bound : tc_bound{};
   CUtensorMap mA  = make_plane_map(a_hi, a_rows_pad, Kp);
   CUtensorMap mB  = make_plane_map(b_hi, b_rows_pad, Kp);
   CUtensorMap mAl = passes >= 2 ? make_plane_map(a_lo, a_rows_pad, Kp) : mA;

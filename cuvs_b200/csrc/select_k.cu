@@ -15,7 +15,6 @@
 
 #include <algorithm>
 #include <cfloat>
-#include <cstdlib>
 
 namespace b200 {
 namespace {
@@ -256,7 +255,7 @@ __global__ void __launch_bounds__(kRegThreads, E <= 32 ? 2 : 1) select_k_reg_ker
   // about 1 % .. 3 % of the row lies below T, of which the k-th smallest is one with overwhelming probability (k = 48,
   // len = 16384: miss rate ~ 4e-5 on exchangeable data).  The first binning round then only counts keys <= T; if fewer than
   // `need` keys are there (adversarial order, e.g. a sorted row) the round is repeated over the full span — exactness never
-  // depends on the sample.  CUVS_B200_SELECT_NOSAMPLE=1 (read by the launcher: sample_elems = 0) turns it off.
+  // depends on the sample.
   if (sample_elems > 0) {
     uint32_t smin = 0xffffffffu;
 #pragma unroll
@@ -368,7 +367,7 @@ template <typename IdxIn, typename IdxOut, bool HasIdx>
 void launch(cudaStream_t stream, const float* in_val, const void* in_idx, int64_t batch, int64_t len, int64_t in_ld,
             int k, float* out_val, void* out_idx, bool select_min)
 {
-  if (len >= 2048 && len <= 64 * kRegThreads && k <= kRegMaxK && getenv("CUVS_B200_SELECT_RADIX") == nullptr) {
+  if (len >= 2048 && len <= 64 * kRegThreads && k <= kRegMaxK) {
     count_launch();
     const unsigned grid = static_cast<unsigned>(batch);
     static bool carve = [] {  // two resident CTAs need ~40 KB of shared memory: ask for the carve-out once per instantiation
@@ -382,8 +381,7 @@ void launch(cudaStream_t stream, const float* in_val, const void* in_idx, int64_
     auto ii = static_cast<const IdxIn*>(in_idx);
     auto oo = static_cast<IdxOut*>(out_idx);
     // sample elements per thread for the kernel's sampled bound: 32 * es ~ 0.7 * len / k samples per warp (0 = no sampling)
-    static const bool no_sample = getenv("CUVS_B200_SELECT_NOSAMPLE") != nullptr;
-    const int es = no_sample ? 0 : static_cast<int>(std::min<int64_t>(64, (7 * len) / (320 * static_cast<int64_t>(std::max(k, 1)))));
+    const int es = static_cast<int>(std::min<int64_t>(64, (7 * len) / (320 * static_cast<int64_t>(std::max(k, 1)))));
     if (len <= 8 * kRegThreads) select_k_reg_kernel<8, IdxIn, IdxOut, HasIdx><<<grid, kRegThreads, 0, stream>>>(in_val, ii, len, in_ld, k, out_val, oo, select_min, es);
     else if (len <= 16 * kRegThreads) select_k_reg_kernel<16, IdxIn, IdxOut, HasIdx><<<grid, kRegThreads, 0, stream>>>(in_val, ii, len, in_ld, k, out_val, oo, select_min, es);
     else if (len <= 32 * kRegThreads) select_k_reg_kernel<32, IdxIn, IdxOut, HasIdx><<<grid, kRegThreads, 0, stream>>>(in_val, ii, len, in_ld, k, out_val, oo, select_min, es);

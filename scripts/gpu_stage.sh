@@ -21,7 +21,6 @@ for stage in "$@"; do
     profcagra)  CUVS_B200_PROFILE=1 timeout 900 ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:cagra_search -c 1 -f -o gpurun_out/r02_cagra python bench.py --workload cagra --steps 1 --no-cpu > gpurun_out/profcagra.log 2>&1; echo "profcagra rc=$?" ;;
     profc2tc)   CUVS_B200_PROFILE=1 timeout 900 ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:tc_scan_kernel -c 2 -f -o gpurun_out/r02_c2 python bench.py --workload ivf_pq_c2 --steps 1 --no-cpu --no-aux > gpurun_out/profc2tc.log 2>&1; echo "profc2tc rc=$?" ;;
     launchesc2) CUVS_B200_PROFILE=1 timeout 900 ncu --profile-from-start off --metrics gpu__time_duration.sum --clock-control none --csv --log-file gpurun_out/r02_launchesc2.csv python bench.py --workload ivf_pq_c2 --steps 1 --no-cpu --no-aux > gpurun_out/launchesc2.log 2>&1; echo "launchesc2 rc=$?" ;;
-    abcagra)    timeout 600 python scripts/ab_cagra.py > gpurun_out/ab_cagra.log 2>&1; echo "abcagra rc=$?" ;;
     cagra_tests) timeout 600 python -m pytest tests/test_cagra_gpu.py -q > gpurun_out/cagra_tests.log 2>&1; echo "cagra_tests rc=$?" ;;
     profselect) CUVS_B200_PROFILE=1 timeout 900 ncu --profile-from-start off --set full --clock-control none --import-source on -k regex:select_k_reg -c 1 -f -o gpurun_out/r02_selectk python scripts/sweep_probes.py 100000000 16384 "48" > gpurun_out/profselect.log 2>&1; echo "profselect rc=$?" ;;
     benchq)     timeout 900 python bench.py --no-cpu --no-aux > gpurun_out/bench_quick.log 2>&1; echo "benchq rc=$?" ;;
