@@ -8,6 +8,7 @@
 
 #include <algorithm>
 #include <cfloat>
+#include <cmath>
 #include <vector>
 
 namespace b200 {
@@ -634,6 +635,47 @@ void assign_nearest(resources* res, const __nv_bfloat16* x_hi, const __nv_bfloat
                                                                scores ? scores + r0 : nullptr);
     B2_CUDA(cudaGetLastError());
   }
+}
+
+void label_rows(resources* res, const tc_rows& centers, const float* x, int64_t n, int d, const float* row_scale, uint32_t* labels)
+{
+  tc_rows_tmp xp;
+  xp.build(res->stream, x, n, d, true, 0, row_scale);
+  assign_nearest(res, xp.hi.data(), xp.lo.data(), n, xp.rows_pad, xp.Kp, centers, labels, nullptr);
+}
+
+int64_t training_subsample(cudaStream_t s, const float* x, int64_t n, int d, uint32_t n_lists, double fraction, dbuf<float>& out)
+{
+  // the reference's rule: ivf_flat_build.cuh:430-455
+  fraction             = std::min(1.0, std::max(fraction, 0.0));
+  int64_t n_train      = std::max<int64_t>(n_lists, std::min<int64_t>(n, static_cast<int64_t>(std::llround(n * fraction))));
+  n_train              = std::min<int64_t>(n_train, std::max<int64_t>(static_cast<int64_t>(n_lists) * 1024, 1 << 18));
+  n_train              = std::min(n_train, n);
+  const int64_t stride = std::max<int64_t>(1, n / n_train);
+  n_train              = std::min(n_train, (n + stride - 1) / stride);
+  out.alloc(static_cast<size_t>(n_train) * d, s);
+  B2_CUDA(cudaMemcpy2DAsync(out.data(), sizeof(float) * d, x, sizeof(float) * d * stride, sizeof(float) * d, n_train,
+                            cudaMemcpyDefault, s));
+  return n_train;
+}
+
+const int64_t* extend_args(resources* res, DLManagedTensor* new_vectors, DLManagedTensor* new_indices, int dim, f32_matrix& v,
+                           dbuf<int64_t>& ids_buf)
+{
+  B2_EXPECTS(new_vectors != nullptr, "new_vectors is null");
+  const DLTensor& nv = new_vectors->dl_tensor;
+  B2_EXPECTS(dl_is_dataset_dtype(nv), "Unsupported new_vectors DLtensor dtype: %d and bits: %d", nv.dtype.code, nv.dtype.bits);
+  widen_to_f32(res, nv, v);
+  B2_EXPECTS(dl_is(v.t, kDLFloat, 32) && v.t.ndim == 2 && v.t.shape[1] == dim && dl_is_c_contiguous(v.t),
+             "new_vectors must be [n, dim] row-major");
+  if (!new_indices) return nullptr;
+  const int64_t n    = v.t.shape[0];
+  const DLTensor& it = new_indices->dl_tensor;
+  B2_EXPECTS(dl_is(it, kDLInt, 64) && it.shape[0] == n, "new_indices must be int64 [n]");
+  if (dl_is_device(it) && it.device.device_type != kDLCUDAHost) return dl_ptr<int64_t>(it);
+  ids_buf.alloc(static_cast<size_t>(n), res->stream);
+  B2_CUDA(cudaMemcpyAsync(ids_buf.data(), dl_ptr<int64_t>(it), sizeof(int64_t) * n, cudaMemcpyHostToDevice, res->stream));
+  return ids_buf.data();
 }
 
 void bucket_probes(resources* res, const uint32_t* probes, int64_t nq, int n_probes, int64_t n_lists,

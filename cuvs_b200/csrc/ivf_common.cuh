@@ -48,6 +48,21 @@ void coarse_select(resources* res, const tc_rows_tmp& queries, const tc_rows& ce
 /** labels[i] = argmin_j (hn[j] - x_i . c_j)  (nearest centre, approx = fp32-grade split products); optional score out. */
 void assign_nearest(resources* res, const __nv_bfloat16* x_hi, const __nv_bfloat16* x_lo, int64_t n, int64_t x_rows_pad,
                     int Kp, const tc_rows& centers, uint32_t* labels, float* scores /*nullable*/);
+/** labels[i] = nearest centre of the device rows x [n, d], each row scaled by row_scale[i] first (nullable). */
+void label_rows(resources* res, const tc_rows& centers, const float* x, int64_t n, int d, const float* row_scale, uint32_t* labels);
+
+/**
+ * Coarse training set of an IVF build: an evenly strided subsample of the dataset x [n, d] (host or device) with about
+ * n * fraction rows, at least n_lists and at most max(1024 n_lists, 2^18).  Fills `out` and returns its row count.
+ */
+int64_t training_subsample(cudaStream_t s, const float* x, int64_t n, int d, uint32_t n_lists, double fraction, dbuf<float>& out);
+
+/**
+ * Arguments of an IVF Extend call: checks new_vectors and widens it to fp32 rows [n, dim] in `v`, checks new_indices and
+ * returns it as device int64 [n] (host ids are staged into `ids_buf`), or null when no ids are given.
+ */
+const int64_t* extend_args(resources* res, DLManagedTensor* new_vectors, DLManagedTensor* new_indices, int dim, f32_matrix& v,
+                           dbuf<int64_t>& ids_buf);
 
 /**
  * (query, probe) pairs bucketed by list, on the device.

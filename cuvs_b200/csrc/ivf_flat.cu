@@ -56,25 +56,6 @@ struct ivf_flat_index {
 
 namespace {
 
-__global__ void scatter_rows_kernel(const float* __restrict__ src, int64_t n, int d, const int64_t* __restrict__ dst_rows,
-                                    const int64_t* __restrict__ src_ids, int64_t id0, float* __restrict__ dst,
-                                    int64_t* __restrict__ dst_ids)
-{
-  int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (t >= n * d) return;
-  int64_t r = t / d;
-  int c     = static_cast<int>(t % d);
-  int64_t o = dst_rows[r];
-  dst[o * d + c] = src[t];
-  if (c == 0) dst_ids[o] = src_ids ? src_ids[r] : id0 + r;
-}
-
-__global__ void fill_i64_kernel(int64_t* p, int64_t n, int64_t v)
-{
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i < n) p[i] = v;
-}
-
 __global__ void half_norms_masked_kernel(const float* __restrict__ xn, const int64_t* __restrict__ ids, int64_t n, bool zero,
                                          float* __restrict__ hn)
 {
@@ -99,30 +80,6 @@ __global__ void rsqrt_rows_kernel(const float* __restrict__ xn, float* __restric
 {
   int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
   if (i < n) out[i] = xn[i] > 0.f ? 1.0f / sqrtf(xn[i]) : 0.f;
-}
-
-// positions of old rows in the new layout (same order inside each list)
-__global__ void remap_old_rows_kernel(const int64_t* __restrict__ old_off, const int64_t* __restrict__ new_off,
-                                      const uint32_t* __restrict__ old_sizes, int64_t n_lists, int64_t* __restrict__ dst_rows,
-                                      int64_t old_rows_total)
-{
-  // one CTA per list
-  int64_t l = blockIdx.x;
-  if (l >= n_lists) return;
-  for (uint32_t i = threadIdx.x; i < old_sizes[l]; i += blockDim.x) dst_rows[old_off[l] + i] = new_off[l] + i;
-}
-
-__global__ void move_rows_kernel(const float* __restrict__ src, const int64_t* __restrict__ src_ids, int64_t rows, int d,
-                                 const int64_t* __restrict__ dst_rows, float* __restrict__ dst, int64_t* __restrict__ dst_ids)
-{
-  int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (t >= rows * d) return;
-  int64_t r = t / d;
-  if (src_ids[r] == kPadId) return;  // padding row of the old layout
-  int c     = static_cast<int>(t % d);
-  int64_t o = dst_rows[r];
-  dst[o * d + c] = src[t];
-  if (c == 0) dst_ids[o] = src_ids[r];
 }
 
 void refresh_tc_side(resources* res, ivf_flat_index& idx)
@@ -163,74 +120,27 @@ void refresh_centers_tc(resources* res, ivf_flat_index& idx)
   idx.centers_tc.build(s, idx.centers.data(), idx.n_lists, idx.dim, is_l2(idx.metric) ? cn.data() : nullptr, true, scale.data());
 }
 
-// Append rows (device, row-major) with the given ids (device int64 or null => id0 + i).
-void ivf_flat_extend(resources* res, ivf_flat_index& idx, const float* x, int64_t n, const int64_t* new_ids, int64_t id0)
+// Append the rows of `t` (host or device, row-major fp32) with the given ids (device int64 or null => id0 + i).
+void ivf_flat_extend(resources* res, ivf_flat_index& idx, const DLTensor& t, const int64_t* new_ids, int64_t id0)
 {
   auto s = res->stream;
-  if (n == 0) return;
-  // 1. nearest centre of every new row
-  tc_rows_tmp xp;
-  dbuf<float> scale;
-  if (idx.metric == CosineExpanded) {
-    dbuf<float> xn(static_cast<size_t>(n), s);
-    row_norms(s, x, n, idx.dim, idx.dim, xn.data());
-    scale.alloc(static_cast<size_t>(n), s);
-    count_launch();
-    rsqrt_rows_kernel<<<blocks_for(n, 256), 256, 0, s>>>(xn.data(), scale.data(), n);
-  }
-  xp.build(s, x, n, idx.dim, true, 0, scale.data());
-  dbuf<uint32_t> labels(static_cast<size_t>(n), s);
-  assign_nearest(res, xp.hi.data(), xp.lo.data(), n, xp.rows_pad, xp.Kp, idx.centers_tc, labels.data(), nullptr);
-  // 2. new layout = old sizes + new counts
-  std::vector<int64_t> add = count_labels(s, labels.data(), n, idx.n_lists);
-  std::vector<int64_t> old_sizes = idx.lists.h_sizes.empty() ? std::vector<int64_t>(idx.n_lists, 0) : idx.lists.h_sizes;
-  std::vector<int64_t> sizes(idx.n_lists);
-  for (uint32_t l = 0; l < idx.n_lists; ++l) sizes[l] = old_sizes[l] + add[l];
-  list_layout nl;
-  nl.set_sizes(s, sizes);
-  owned<float> ndata(static_cast<size_t>(std::max<int64_t>(nl.rows_total, 1)) * idx.dim);
-  owned<int64_t> nids(static_cast<size_t>(std::max<int64_t>(nl.rows_total, 1)));
-  B2_CUDA(cudaMemsetAsync(ndata.data(), 0, sizeof(float) * static_cast<size_t>(nl.rows_total) * idx.dim, s));
-  count_launch();
-  fill_i64_kernel<<<blocks_for(nl.rows_total, 256), 256, 0, s>>>(nids.data(), nl.rows_total, kPadId);
-  // 3. move the old rows
-  if (idx.lists.rows_total > 0) {
-    dbuf<int64_t> dst_old(static_cast<size_t>(idx.lists.rows_total), s);
-    count_launch(2);
-    remap_old_rows_kernel<<<idx.n_lists, 128, 0, s>>>(idx.lists.d_offsets.data(), nl.d_offsets.data(), idx.lists.d_sizes.data(),
-                                                       idx.n_lists, dst_old.data(), idx.lists.rows_total);
-    move_rows_kernel<<<blocks_for(idx.lists.rows_total * idx.dim, 256), 256, 0, s>>>(
-      idx.data.data(), idx.ids.data(), idx.lists.rows_total, idx.dim, dst_old.data(), ndata.data(), nids.data());
-    B2_CUDA(cudaGetLastError());
-  }
-  // 4. scatter the new rows behind them
-  dbuf<int64_t> dst_new(static_cast<size_t>(n), s);
-  place_rows(s, labels.data(), n, nl, old_sizes, dst_new.data());
-  count_launch();
-  scatter_rows_kernel<<<blocks_for(n * idx.dim, 256), 256, 0, s>>>(x, n, idx.dim, dst_new.data(), new_ids, id0, ndata.data(),
-                                                                    nids.data());
-  B2_CUDA(cudaGetLastError());
-  B2_CUDA(cudaStreamSynchronize(s));
-  idx.data  = std::move(ndata);
-  idx.ids   = std::move(nids);
-  idx.lists = std::move(nl);
+  if (t.shape[0] == 0) return;
+  auto label = [&](const float* x, int64_t n, uint32_t* labels) {
+    dbuf<float> scale;
+    if (idx.metric == CosineExpanded) {
+      dbuf<float> xn(static_cast<size_t>(n), s);
+      row_norms(s, x, n, idx.dim, idx.dim, xn.data());
+      scale.alloc(static_cast<size_t>(n), s);
+      count_launch();
+      rsqrt_rows_kernel<<<blocks_for(n, 256), 256, 0, s>>>(xn.data(), scale.data(), n);
+    }
+    label_rows(res, idx.centers_tc, x, n, idx.dim, scale.data(), labels);
+  };
+  auto write = [&](const float* x, int64_t n, const uint32_t*, const int64_t* dst_rows, float* data) {
+    scatter_rows(s, x, n, idx.dim, dst_rows, data);
+  };
+  insert_rows(res, idx.lists, idx.data, idx.dim, idx.ids, t, idx.dim, new_ids, id0, label, write);
   refresh_tc_side(res, idx);
-}
-
-// dataset may live on the host: stage it through the device in chunks
-template <typename Fn>
-void for_device_chunks(resources* res, const DLTensor& t, int d, Fn&& fn)
-{
-  const int64_t n = t.shape[0];
-  const float* p  = dl_ptr<float>(t);
-  if (dl_is_device(t) && t.device.device_type != kDLCUDAHost) { fn(p, n, int64_t(0)); return; }
-  const int64_t chunk = std::max<int64_t>(1, (int64_t(1) << 28) / std::max(d, 1));  // 1 GiB of floats
-  dbuf<float> buf(static_cast<size_t>(std::min(n, chunk)) * d, res->stream);
-  for (int64_t r0 = 0; r0 < n; r0 += chunk) {
-    int64_t rows = std::min(chunk, n - r0);
-    B2_CUDA(cudaMemcpyAsync(buf.data(), p + r0 * d, sizeof(float) * rows * d, cudaMemcpyHostToDevice, res->stream));
-    fn(buf.data(), rows, r0);
-  }
 }
 
 ivf_flat_index* ivf_flat_build(resources* res, const cuvsIvfFlatIndexParams& p, const DLTensor& ds)
@@ -254,28 +164,16 @@ ivf_flat_index* ivf_flat_build(resources* res, const cuvsIvfFlatIndexParams& p, 
   idx->kmeans_trainset_fraction = p.kmeans_trainset_fraction;
   auto s = res->stream;
 
-  // ---- training set: evenly strided subsample (ivf_flat_build.cuh:430-455 uses the same rule)
-  double frac      = std::min(1.0, std::max(p.kmeans_trainset_fraction, 0.0));
-  int64_t n_train  = std::max<int64_t>(p.n_lists, std::min<int64_t>(n, static_cast<int64_t>(std::llround(n * frac))));
-  n_train          = std::min<int64_t>(n_train, std::max<int64_t>(static_cast<int64_t>(p.n_lists) * 1024, 1 << 18));
-  n_train          = std::min(n_train, n);
-  const int64_t stride = std::max<int64_t>(1, n / n_train);
-  n_train          = std::min(n_train, (n + stride - 1) / stride);
-  dbuf<float> train(static_cast<size_t>(n_train) * d, s);
-  B2_CUDA(cudaMemcpy2DAsync(train.data(), sizeof(float) * d, dl_ptr<float>(ds), sizeof(float) * d * stride, sizeof(float) * d,
-                            n_train, cudaMemcpyDefault, s));
-  dbuf<float> train_scaled;
-  const float* train_ptr = train.data();
+  dbuf<float> train;
+  const int64_t n_train = training_subsample(s, dl_ptr<float>(ds), n, d, p.n_lists, p.kmeans_trainset_fraction, train);
   idx->centers.alloc(static_cast<size_t>(p.n_lists) * d);
-  kmeans_train(res, train_ptr, n_train, d, p.n_lists, std::max<uint32_t>(p.kmeans_n_iters, 1), idx->centers.data(), true, true,
+  kmeans_train(res, train.data(), n_train, d, p.n_lists, std::max<uint32_t>(p.kmeans_n_iters, 1), idx->centers.data(), true, true,
                nullptr, nullptr);
   refresh_centers_tc(res, *idx);
   std::vector<int64_t> zero(p.n_lists, 0);
   idx->lists.set_sizes(s, zero);
   refresh_tc_side(res, *idx);
-  if (p.add_data_on_build) {
-    for_device_chunks(res, ds, d, [&](const float* x, int64_t rows, int64_t r0) { ivf_flat_extend(res, *idx, x, rows, nullptr, r0); });
-  }
+  if (p.add_data_on_build) ivf_flat_extend(res, *idx, ds, nullptr, 0);
   return idx.release();
 }
 
@@ -536,34 +434,10 @@ cuvsError_t cuvsIvfFlatExtend(cuvsResources_t res, DLManagedTensor* new_vectors,
   return guarded([=] {
     auto r    = as_res(res);
     auto& idx = flat_of(index);
-    B2_EXPECTS(new_vectors != nullptr, "new_vectors is null");
-    B2_EXPECTS(dl_is_dataset_dtype(new_vectors->dl_tensor), "Unsupported new_vectors DLtensor dtype: %d and bits: %d",
-               new_vectors->dl_tensor.dtype.code, new_vectors->dl_tensor.dtype.bits);
-    f32_matrix wv;
-    widen_to_f32(r, new_vectors->dl_tensor, wv);
-    const DLTensor& v = wv.t;
-    B2_EXPECTS(dl_is(v, kDLFloat, 32) && v.ndim == 2 && v.shape[1] == idx.dim && dl_is_c_contiguous(v), "new_vectors must be [n, dim] row-major");
-    const int64_t n = v.shape[0];
-    dbuf<int64_t> ids_dev;
-    const int64_t* ids = nullptr;
-    if (new_indices) {
-      const DLTensor& it = new_indices->dl_tensor;
-      B2_EXPECTS(dl_is(it, kDLInt, 64) && it.shape[0] == n, "new_indices must be int64 [n]");
-      if (dl_is_device(it) && it.device.device_type != kDLCUDAHost) ids = dl_ptr<int64_t>(it);
-      else {
-        ids_dev.alloc(static_cast<size_t>(n), r->stream);
-        B2_CUDA(cudaMemcpyAsync(ids_dev.data(), dl_ptr<int64_t>(it), sizeof(int64_t) * n, cudaMemcpyHostToDevice, r->stream));
-        ids = ids_dev.data();
-      }
-    }
-    const int64_t id0 = idx.lists.size;  // reference: new ids continue after the current size when none are given
-    if (dl_is_device(v) && v.device.device_type != kDLCUDAHost) {
-      ivf_flat_extend(r, idx, dl_ptr<float>(v), n, ids, id0);
-    } else {
-      dbuf<float> buf(static_cast<size_t>(n) * idx.dim, r->stream);
-      B2_CUDA(cudaMemcpyAsync(buf.data(), dl_ptr<float>(v), sizeof(float) * n * idx.dim, cudaMemcpyHostToDevice, r->stream));
-      ivf_flat_extend(r, idx, buf.data(), n, ids, id0);
-    }
+    f32_matrix v;
+    dbuf<int64_t> ids_buf;
+    const int64_t* ids = extend_args(r, new_vectors, new_indices, idx.dim, v, ids_buf);
+    ivf_flat_extend(r, idx, v.t, ids, idx.lists.size);  // reference: new ids continue after the current size when none are given
   });
 }
 
@@ -673,11 +547,7 @@ cuvsError_t cuvsIvfFlatDeserialize(cuvsResources_t res, const char* filename, cu
     idx->lists.set_sizes(r->stream, sizes);
     B2_EXPECTS(idx->lists.size == n_rows, "ivf_flat::deserialize: list sizes sum to %lld, header says %lld rows", (long long)idx->lists.size,
                (long long)n_rows);
-    const int64_t R = idx->lists.rows_total;
-    idx->data.alloc(static_cast<size_t>(std::max<int64_t>(R, 1)) * idx->dim);
-    idx->ids.alloc(static_cast<size_t>(std::max<int64_t>(R, 1)));
-    B2_CUDA(cudaMemsetAsync(idx->data.data(), 0, sizeof(float) * static_cast<size_t>(R) * idx->dim, r->stream));
-    if (R) fill_i64_kernel<<<blocks_for(R, 256), 256, 0, r->stream>>>(idx->ids.data(), R, kPadId);
+    alloc_padded(r->stream, idx->lists.rows_total, idx->dim, idx->data, idx->ids);
     std::vector<float> rows, inter;
     std::vector<int64_t> ids;
     const int dim = idx->dim, vl = flat_veclen(dim);

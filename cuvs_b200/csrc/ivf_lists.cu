@@ -40,6 +40,33 @@ __global__ void place_rows_kernel(const uint32_t* __restrict__ sorted, const uin
   const uint32_t l = sorted[p];
   dst[order[p]]    = offsets[l] + base_fill[l] + (p - start[l]);
 }
+__global__ void fill_pad_ids_kernel(int64_t* __restrict__ ids, int64_t n)
+{
+  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (i < n) ids[i] = kPadId;
+}
+// one CTA per list
+__global__ void remap_rows_kernel(const int64_t* __restrict__ from_off, const uint32_t* __restrict__ from_sizes,
+                                  const int64_t* __restrict__ to_off, int64_t* __restrict__ dst_rows)
+{
+  const int64_t l = blockIdx.x, o = from_off[l], rows = from_off[l + 1] - o;
+  for (int64_t i = threadIdx.x; i < rows; i += blockDim.x) dst_rows[o + i] = i < from_sizes[l] ? to_off[l] + i : -1;
+}
+template <typename T>
+__global__ void scatter_rows_kernel(const T* __restrict__ src, int64_t rows, int row_elems, const int64_t* __restrict__ dst_rows,
+                                    T* __restrict__ dst)
+{
+  int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (t >= rows * row_elems) return;
+  const int64_t o = dst_rows[t / row_elems];
+  if (o >= 0) dst[o * row_elems + t % row_elems] = src[t];
+}
+__global__ void store_ids_kernel(const int64_t* __restrict__ dst_rows, int64_t n, const int64_t* __restrict__ new_ids, int64_t id0,
+                                 int64_t* __restrict__ ids)
+{
+  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
+  if (i < n) ids[dst_rows[i]] = new_ids ? new_ids[i] : id0 + i;
+}
 }  // namespace
 
 void iota_u32(cudaStream_t s, dbuf<uint32_t>& v, int64_t n)
@@ -123,6 +150,46 @@ void place_rows(cudaStream_t s, const uint32_t* labels, int64_t n, const list_la
                                                                              layout.d_offsets.data(), fill.data(), dst_rows);
   B2_CUDA(cudaGetLastError());
   B2_CUDA(cudaStreamSynchronize(s));  // base_fill is a host vector owned by the caller
+}
+
+template <typename T>
+void alloc_padded(cudaStream_t s, int64_t rows, int row_elems, owned<T>& payload, owned<int64_t>& ids)
+{
+  payload.alloc(static_cast<size_t>(std::max<int64_t>(rows, 1)) * row_elems);
+  ids.alloc(static_cast<size_t>(std::max<int64_t>(rows, 1)));
+  B2_CUDA(cudaMemsetAsync(payload.data(), 0, sizeof(T) * static_cast<size_t>(rows) * row_elems, s));
+  if (rows == 0) return;
+  count_launch();
+  fill_pad_ids_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(ids.data(), rows);
+  B2_CUDA(cudaGetLastError());
+}
+template void alloc_padded<float>(cudaStream_t, int64_t, int, owned<float>&, owned<int64_t>&);
+template void alloc_padded<uint8_t>(cudaStream_t, int64_t, int, owned<uint8_t>&, owned<int64_t>&);
+
+void remap_rows(cudaStream_t s, const list_layout& from, const list_layout& to, int64_t* dst_rows)
+{
+  count_launch();
+  remap_rows_kernel<<<static_cast<unsigned>(from.n_lists), 128, 0, s>>>(from.d_offsets.data(), from.d_sizes.data(),
+                                                                         to.d_offsets.data(), dst_rows);
+  B2_CUDA(cudaGetLastError());
+}
+
+template <typename T>
+void scatter_rows(cudaStream_t s, const T* src, int64_t rows, int row_elems, const int64_t* dst_rows, T* dst)
+{
+  count_launch();
+  scatter_rows_kernel<T><<<blocks_for(rows * row_elems, 256), 256, 0, s>>>(src, rows, row_elems, dst_rows, dst);
+  B2_CUDA(cudaGetLastError());
+}
+template void scatter_rows<float>(cudaStream_t, const float*, int64_t, int, const int64_t*, float*);
+template void scatter_rows<uint8_t>(cudaStream_t, const uint8_t*, int64_t, int, const int64_t*, uint8_t*);
+template void scatter_rows<int64_t>(cudaStream_t, const int64_t*, int64_t, int, const int64_t*, int64_t*);
+
+void store_ids(cudaStream_t s, const int64_t* dst_rows, int64_t n, const int64_t* new_ids, int64_t id0, int64_t* ids)
+{
+  count_launch();
+  store_ids_kernel<<<blocks_for(n, 256), 256, 0, s>>>(dst_rows, n, new_ids, id0, ids);
+  B2_CUDA(cudaGetLastError());
 }
 
 }  // namespace b200

@@ -285,40 +285,6 @@ __global__ void pq_decode_kernel(const uint8_t* __restrict__ codes, const int64_
   if (lane == 0) hn[r] = pad ? INFINITY : (ip ? 0.f : 0.5f * nrm);
 }
 
-__global__ void move_codes_kernel(const uint8_t* __restrict__ src, const int64_t* __restrict__ src_ids, int64_t rows, int pq_dim,
-                                  const int64_t* __restrict__ dst_rows, uint8_t* __restrict__ dst, int64_t* __restrict__ dst_ids)
-{
-  int64_t t = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (t >= rows * pq_dim) return;
-  int64_t r = t / pq_dim;
-  if (src_ids[r] == kPadId) return;
-  int c     = static_cast<int>(t % pq_dim);
-  int64_t o = dst_rows[r];
-  dst[o * pq_dim + c] = src[t];
-  if (c == 0) dst_ids[o] = src_ids[r];
-}
-
-__global__ void remap_rows_kernel(const int64_t* __restrict__ old_off, const int64_t* __restrict__ new_off,
-                                  const uint32_t* __restrict__ old_sizes, int64_t n_lists, int64_t* __restrict__ dst_rows)
-{
-  int64_t l = blockIdx.x;
-  if (l >= n_lists) return;
-  for (uint32_t i = threadIdx.x; i < old_sizes[l]; i += blockDim.x) dst_rows[old_off[l] + i] = new_off[l] + i;
-}
-
-__global__ void set_ids_kernel(const int64_t* __restrict__ dst_rows, const int64_t* __restrict__ src_ids, int64_t id0, int64_t n,
-                               int64_t* __restrict__ ids)
-{
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i < n) ids[dst_rows[i]] = src_ids ? src_ids[i] : id0 + i;
-}
-
-__global__ void fill_i64_kernel(int64_t* p, int64_t n, int64_t v)
-{
-  int64_t i = blockIdx.x * static_cast<int64_t>(blockDim.x) + threadIdx.x;
-  if (i < n) p[i] = v;
-}
-
 __global__ void make_centers_ext_kernel(const float* __restrict__ centers, int64_t n_lists, int dim, int dim_ext,
                                         float* __restrict__ ext)
 {
@@ -570,6 +536,27 @@ void rotate_rows(cudaStream_t s, const float* x, int64_t n, int dim, const float
   }
 }
 
+// Residuals R x - c_rot[label] [n, rot_dim] of the device rows x [n, dim]; when `codes` is given, also the nearest PQ code of
+// every (row, subspace), stored at codes[(dst_rows ? dst_rows[i] : i) * pq_dim + subspace].
+dbuf<float> encode_rows(resources* res, const ivf_pq_index& idx, const float* x, int64_t n, const uint32_t* labels,
+                        uint8_t* codes = nullptr, const int64_t* dst_rows = nullptr)
+{
+  auto s = res->stream;
+  dbuf<float> xr(static_cast<size_t>(n) * idx.rot_dim, s), rs(static_cast<size_t>(n) * idx.rot_dim, s);
+  rotate_rows(s, x, n, idx.dim, idx.rotation.data(), idx.rot_dim, xr.data());
+  count_launch();
+  residual_kernel<<<blocks_for(n * idx.rot_dim, 256), 256, 0, s>>>(xr.data(), labels, idx.centers_rot.data(), n, idx.rot_dim, rs.data());
+  if (codes) {
+    const size_t smem = static_cast<size_t>(idx.pq_len) * idx.book() * sizeof(float);
+    count_launch();
+    pq_assign_kernel<<<dim3(blocks_for(n, 128), idx.pq_dim), 128, smem, s>>>(
+      rs.data(), n, idx.rot_dim, idx.pq_dim, idx.pq_len, idx.book(), idx.pq_centers.data(),
+      idx.codebook_kind == CUVS_IVF_PQ_CODEBOOK_GEN_PER_CLUSTER, labels, codes, dst_rows);
+  }
+  B2_CUDA(cudaGetLastError());
+  return rs;
+}
+
 void refresh_centers(resources* res, ivf_pq_index& idx)
 {
   auto s = res->stream;
@@ -668,87 +655,17 @@ void train_codebooks(resources* res, ivf_pq_index& idx, const float* resid, cons
   }
 }
 
-// rows of `t` in device-resident chunks of at most 512 MiB (host tensors are staged through one reusable buffer)
-template <typename Fn>
-void for_device_chunks(resources* res, const DLTensor& t, int d, Fn&& fn)
-{
-  const int64_t n = t.shape[0];
-  const float* p  = dl_ptr<float>(t);
-  const int64_t chunk = std::max<int64_t>(1, (int64_t(1) << 27) / std::max(d, 1));  // 512 MiB of floats per step
-  const bool dev = dl_is_device(t) && t.device.device_type != kDLCUDAHost;
-  dbuf<float> buf;
-  if (!dev) buf.alloc(static_cast<size_t>(std::min(n, chunk)) * d, res->stream);
-  for (int64_t r0 = 0; r0 < n; r0 += chunk) {
-    int64_t rows = std::min(chunk, n - r0);
-    if (dev) fn(p + r0 * d, rows, r0);
-    else {
-      B2_CUDA(cudaMemcpyAsync(buf.data(), p + r0 * d, sizeof(float) * rows * d, cudaMemcpyHostToDevice, res->stream));
-      fn(buf.data(), rows, r0);
-    }
-  }
-}
-
-// Insert the rows of `t` (ids new_ids[i] or id0 + i).  Two passes over the chunks so that the lists are laid out ONCE for
-// the whole insertion: (1) label every row and count per list, (2) encode every chunk straight into its final place.  The
-// decoded rows are refreshed once at the end.  (Inserting chunk by chunk would re-pack and re-decode the whole index per
-// chunk: quadratic in the index size, minutes at 100M rows.)
+// Insert the rows of `t` (ids new_ids[i] or id0 + i): codes are encoded straight into their place in the new lists, and the
+// decoded rows are refreshed once at the end.
 void ivf_pq_extend(resources* res, ivf_pq_index& idx, const DLTensor& t, const int64_t* new_ids, int64_t id0)
 {
-  auto s          = res->stream;
-  const int64_t n = t.shape[0];
-  if (n == 0) return;
-  dbuf<uint32_t> labels(static_cast<size_t>(n), s);
-  std::vector<int64_t> old_sizes = idx.lists.h_sizes.empty() ? std::vector<int64_t>(idx.n_lists, 0) : idx.lists.h_sizes;
-  std::vector<int64_t> sizes     = old_sizes;
-  std::vector<std::vector<int64_t>> chunk_add;
-  for_device_chunks(res, t, idx.dim, [&](const float* x, int64_t rows, int64_t r0) {
-    tc_rows_tmp xp;
-    xp.build(s, x, rows, idx.dim, true);
-    assign_nearest(res, xp.hi.data(), xp.lo.data(), rows, xp.rows_pad, xp.Kp, idx.centers_tc, labels.data() + r0, nullptr);
-    chunk_add.push_back(count_labels(s, labels.data() + r0, rows, idx.n_lists));
-    for (uint32_t l = 0; l < idx.n_lists; ++l) sizes[l] += chunk_add.back()[l];
-  });
-  list_layout nl;
-  nl.set_sizes(s, sizes);
-  owned<uint8_t> ncodes(static_cast<size_t>(std::max<int64_t>(nl.rows_total, 1)) * idx.pq_dim);
-  owned<int64_t> nids(static_cast<size_t>(std::max<int64_t>(nl.rows_total, 1)));
-  B2_CUDA(cudaMemsetAsync(ncodes.data(), 0, static_cast<size_t>(nl.rows_total) * idx.pq_dim, s));
-  count_launch();
-  fill_i64_kernel<<<blocks_for(nl.rows_total, 256), 256, 0, s>>>(nids.data(), nl.rows_total, kPadId);
-  if (idx.lists.rows_total > 0) {
-    ensure_flat_codes(res, idx);
-    dbuf<int64_t> dst_old(static_cast<size_t>(idx.lists.rows_total), s);
-    count_launch(2);
-    remap_rows_kernel<<<idx.n_lists, 128, 0, s>>>(idx.lists.d_offsets.data(), nl.d_offsets.data(), idx.lists.d_sizes.data(), idx.n_lists,
-                                                   dst_old.data());
-    move_codes_kernel<<<blocks_for(idx.lists.rows_total * idx.pq_dim, 256), 256, 0, s>>>(
-      idx.codes.data(), idx.ids.data(), idx.lists.rows_total, idx.pq_dim, dst_old.data(), ncodes.data(), nids.data());
-    B2_CUDA(cudaGetLastError());
-  }
-  std::vector<int64_t> fill = old_sizes;  // rows already placed in each list
-  size_t ci = 0;
-  for_device_chunks(res, t, idx.dim, [&](const float* x, int64_t rows, int64_t r0) {
-    dbuf<int64_t> dst_new(static_cast<size_t>(rows), s);
-    place_rows(s, labels.data() + r0, rows, nl, fill, dst_new.data());
-    for (uint32_t l = 0; l < idx.n_lists; ++l) fill[l] += chunk_add[ci][l];
-    ++ci;
-    // encode: rotate, residual, nearest code per subspace
-    dbuf<float> xr(static_cast<size_t>(rows) * idx.rot_dim, s), rs(static_cast<size_t>(rows) * idx.rot_dim, s);
-    rotate_rows(s, x, rows, idx.dim, idx.rotation.data(), idx.rot_dim, xr.data());
-    count_launch(3);
-    residual_kernel<<<blocks_for(rows * idx.rot_dim, 256), 256, 0, s>>>(xr.data(), labels.data() + r0, idx.centers_rot.data(), rows,
-                                                                         idx.rot_dim, rs.data());
-    const size_t smem = static_cast<size_t>(idx.pq_len) * idx.book() * sizeof(float);
-    pq_assign_kernel<<<dim3(blocks_for(rows, 128), idx.pq_dim), 128, smem, s>>>(
-      rs.data(), rows, idx.rot_dim, idx.pq_dim, idx.pq_len, idx.book(), idx.pq_centers.data(),
-      idx.codebook_kind == CUVS_IVF_PQ_CODEBOOK_GEN_PER_CLUSTER, labels.data() + r0, ncodes.data(), dst_new.data());
-    set_ids_kernel<<<blocks_for(rows, 256), 256, 0, s>>>(dst_new.data(), new_ids ? new_ids + r0 : nullptr, id0 + r0, rows, nids.data());
-    B2_CUDA(cudaGetLastError());
-  });
-  B2_CUDA(cudaStreamSynchronize(s));
-  idx.codes = std::move(ncodes);
-  idx.ids   = std::move(nids);
-  idx.lists = std::move(nl);
+  if (t.shape[0] == 0) return;
+  if (idx.lists.rows_total > 0) ensure_flat_codes(res, idx);
+  auto label = [&](const float* x, int64_t n, uint32_t* labels) { label_rows(res, idx.centers_tc, x, n, idx.dim, nullptr, labels); };
+  auto write = [&](const float* x, int64_t n, const uint32_t* labels, const int64_t* dst_rows, uint8_t* codes) {
+    encode_rows(res, idx, x, n, labels, codes, dst_rows);
+  };
+  insert_rows(res, idx.lists, idx.codes, idx.pq_dim, idx.ids, t, idx.dim, new_ids, id0, label, write);
   refresh_decoded(res, idx);
 }
 
@@ -785,16 +702,9 @@ ivf_pq_index* ivf_pq_build(resources* res, const cuvsIvfPqIndexParams& p, const 
   init_shape(*idx, p, d);
   auto s = res->stream;
 
-  // training subsample (strided), k-means for the coarse centres
-  double frac     = std::min(1.0, std::max(p.kmeans_trainset_fraction, 0.0));
-  int64_t n_train = std::max<int64_t>(p.n_lists, std::min<int64_t>(n, static_cast<int64_t>(std::llround(n * frac))));
-  n_train         = std::min<int64_t>(n_train, std::max<int64_t>(static_cast<int64_t>(p.n_lists) * 1024, 1 << 18));
-  n_train         = std::min(n_train, n);
-  const int64_t stride = std::max<int64_t>(1, n / n_train);
-  n_train         = std::min(n_train, (n + stride - 1) / stride);
-  dbuf<float> train(static_cast<size_t>(n_train) * d, s);
-  B2_CUDA(cudaMemcpy2DAsync(train.data(), sizeof(float) * d, dl_ptr<float>(ds), sizeof(float) * d * stride, sizeof(float) * d, n_train,
-                            cudaMemcpyDefault, s));
+  // training subsample, k-means for the coarse centres
+  dbuf<float> train;
+  const int64_t n_train = training_subsample(s, dl_ptr<float>(ds), n, d, p.n_lists, p.kmeans_trainset_fraction, train);
   idx->centers.alloc(static_cast<size_t>(p.n_lists) * d);
   kmeans_train(res, train.data(), n_train, d, p.n_lists, std::max<uint32_t>(p.kmeans_n_iters, 1), idx->centers.data(), true, true, nullptr, nullptr);
   refresh_centers(res, *idx);
@@ -812,14 +722,9 @@ ivf_pq_index* ivf_pq_build(resources* res, const cuvsIvfPqIndexParams& p, const 
   if (idx->codebook_kind == CUVS_IVF_PQ_CODEBOOK_GEN_PER_CLUSTER) n_pq = n_train;
   n_pq = std::max<int64_t>(n_pq, std::min<int64_t>(n_train, idx->book()));
   {
-    tc_rows_tmp tp;
-    tp.build(s, train.data(), n_pq, d, true);
     dbuf<uint32_t> labels(static_cast<size_t>(n_pq), s);
-    assign_nearest(res, tp.hi.data(), tp.lo.data(), n_pq, tp.rows_pad, tp.Kp, idx->centers_tc, labels.data(), nullptr);
-    dbuf<float> xr(static_cast<size_t>(n_pq) * idx->rot_dim, s), rs(static_cast<size_t>(n_pq) * idx->rot_dim, s);
-    rotate_rows(s, train.data(), n_pq, d, idx->rotation.data(), idx->rot_dim, xr.data());
-    count_launch();
-    residual_kernel<<<blocks_for(n_pq * idx->rot_dim, 256), 256, 0, s>>>(xr.data(), labels.data(), idx->centers_rot.data(), n_pq, idx->rot_dim, rs.data());
+    label_rows(res, idx->centers_tc, train.data(), n_pq, d, nullptr, labels.data());
+    dbuf<float> rs = encode_rows(res, *idx, train.data(), n_pq, labels.data());
     train_codebooks(res, *idx, rs.data(), labels.data(), n_pq, std::max<uint32_t>(p.kmeans_n_iters, 1));
   }
   std::vector<int64_t> zero(p.n_lists, 0);
@@ -1269,28 +1174,10 @@ cuvsError_t cuvsIvfPqExtend(cuvsResources_t res, DLManagedTensor* new_vectors, D
   return guarded([=] {
     auto r    = as_res(res);
     auto& idx = pq_of(index);
-    B2_EXPECTS(new_vectors != nullptr, "new_vectors is null");
-    B2_EXPECTS(dl_is_dataset_dtype(new_vectors->dl_tensor), "Unsupported new_vectors DLtensor dtype: %d and bits: %d",
-               new_vectors->dl_tensor.dtype.code, new_vectors->dl_tensor.dtype.bits);
-    f32_matrix wv;
-    widen_to_f32(r, new_vectors->dl_tensor, wv);
-    const DLTensor& v = wv.t;
-    B2_EXPECTS(dl_is(v, kDLFloat, 32) && v.ndim == 2 && v.shape[1] == idx.dim && dl_is_c_contiguous(v), "new_vectors must be [n, dim] row-major");
-    const int64_t n = v.shape[0];
-    dbuf<int64_t> ids_dev;
-    const int64_t* ids = nullptr;
-    if (new_indices) {
-      const DLTensor& it = new_indices->dl_tensor;
-      B2_EXPECTS(dl_is(it, kDLInt, 64) && it.shape[0] == n, "new_indices must be int64 [n]");
-      if (dl_is_device(it) && it.device.device_type != kDLCUDAHost) ids = dl_ptr<int64_t>(it);
-      else {
-        ids_dev.alloc(static_cast<size_t>(n), r->stream);
-        B2_CUDA(cudaMemcpyAsync(ids_dev.data(), dl_ptr<int64_t>(it), sizeof(int64_t) * n, cudaMemcpyHostToDevice, r->stream));
-        ids = ids_dev.data();
-      }
-    }
-    const int64_t id0 = idx.lists.size;
-    ivf_pq_extend(r, idx, v, ids, id0);
+    f32_matrix v;
+    dbuf<int64_t> ids_buf;
+    const int64_t* ids = extend_args(r, new_vectors, new_indices, idx.dim, v, ids_buf);
+    ivf_pq_extend(r, idx, v.t, ids, idx.lists.size);
   });
 }
 
@@ -1462,11 +1349,7 @@ cuvsError_t cuvsIvfPqDeserialize(cuvsResources_t res, const char* filename, cuvs
     idx->lists.set_sizes(r->stream, sizes);
     B2_EXPECTS(idx->lists.size == n_rows, "ivf_pq::deserialize: list sizes sum to %lld, header says %lld rows", (long long)idx->lists.size,
                (long long)n_rows);
-    const int64_t R = idx->lists.rows_total;
-    idx->codes.alloc(static_cast<size_t>(std::max<int64_t>(R, 1)) * idx->pq_dim);
-    idx->ids.alloc(static_cast<size_t>(std::max<int64_t>(R, 1)));
-    B2_CUDA(cudaMemsetAsync(idx->codes.data(), 0, static_cast<size_t>(R) * idx->pq_dim, r->stream));
-    if (R) fill_i64_kernel<<<blocks_for(R, 256), 256, 0, r->stream>>>(idx->ids.data(), R, kPadId);
+    alloc_padded(r->stream, idx->lists.rows_total, idx->pq_dim, idx->codes, idx->ids);
     std::vector<uint8_t> packed, codes;
     std::vector<int64_t> ids;
     const int C = 128 / idx->pq_bits;
@@ -1512,18 +1395,10 @@ cuvsError_t cuvsIvfPqTransform(cuvsResources_t res, cuvsIvfPqIndex_t index, DLMa
     B2_EXPECTS(dl_is(oc, kDLUInt, 8) && oc.ndim == 2 && oc.shape[0] == n && oc.shape[1] == out_ld && dl_is_device(oc), "output_dataset must be device uint8 [n, %d]", out_ld);
     if (n == 0) return;
     auto s = r->stream;
-    tc_rows_tmp xp;
-    xp.build(s, dl_ptr<float>(x), n, idx.dim, true);
     uint32_t* labels = dl_ptr<uint32_t>(ol);
-    assign_nearest(r, xp.hi.data(), xp.lo.data(), n, xp.rows_pad, xp.Kp, idx.centers_tc, labels, nullptr);
-    dbuf<float> xr(static_cast<size_t>(n) * idx.rot_dim, s), rs(static_cast<size_t>(n) * idx.rot_dim, s);
-    rotate_rows(s, dl_ptr<float>(x), n, idx.dim, idx.rotation.data(), idx.rot_dim, xr.data());
-    residual_kernel<<<blocks_for(n * idx.rot_dim, 256), 256, 0, s>>>(xr.data(), labels, idx.centers_rot.data(), n, idx.rot_dim, rs.data());
+    label_rows(r, idx.centers_tc, dl_ptr<float>(x), n, idx.dim, nullptr, labels);
     dbuf<uint8_t> codes(static_cast<size_t>(n) * idx.pq_dim, s);
-    const size_t smem = static_cast<size_t>(idx.pq_len) * idx.book() * sizeof(float);
-    pq_assign_kernel<<<dim3(blocks_for(n, 128), idx.pq_dim), 128, smem, s>>>(rs.data(), n, idx.rot_dim, idx.pq_dim, idx.pq_len, idx.book(),
-                                                                               idx.pq_centers.data(), idx.codebook_kind == CUVS_IVF_PQ_CODEBOOK_GEN_PER_CLUSTER,
-                                                                               labels, codes.data(), nullptr);
+    encode_rows(r, idx, dl_ptr<float>(x), n, labels, codes.data());
     pack_codes_kernel<<<blocks_for(n, 128), 128, 0, s>>>(codes.data(), n, idx.pq_dim, idx.pq_bits, out_ld, dl_ptr<uint8_t>(oc));
     B2_CUDA(cudaGetLastError());
   });
